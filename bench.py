@@ -22,6 +22,8 @@ graph launches from one host thread.
             message when the oracle chain fits the CPU budget) + size-independent properties + a full D=4, N=2 step
   cpu_baseline  the numpy oracle (port of the reference path, exact-SVD branch) on this box's host cores, bounded sample
   ite       second headline metric ("ms per ITE step"): one loop body of ite_per_mode, wall clock on rank 0
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 (every unit cell's new messages and errors) as
+DIR/<name>.npy, so that two builds can be compared output for output on the same seeded inputs.
 `--impl reference` times that CPU port as the reference arm: a step there is a BOUNDED SAMPLE (a prefix of one chain's swallow
 order on steady-state messages); value = fraction of a message done / measured seconds, ms_per_step = measured, no extrapolation.
 """
@@ -67,7 +69,11 @@ def parse():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--cpu-budget-s", type=float, default=25.0)
     ap.add_argument("--parity-budget-s", type=float, default=100.0, help="run the full oracle chain for the parity check if it is estimated to fit")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy, float64")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     c = CONFIGS[a.config]
     a.D = c["D"] if a.D is None else a.D
     a.N = c["N"] if a.N is None else a.N
@@ -90,6 +96,41 @@ def workload_name(a):
     n_s = 3 * (3 * a.N * a.N - 3 * a.N + 1)
     return (f"Kagome Heisenberg-PEPS block BP, D={a.D}, block N={a.N} ({n_s} sites, 6 messages x {2 * a.N - 1} MPS sites), "
             f"chi_bp={2 * a.D * a.D}, damping={a.damping}, complex128")
+
+
+DUMP_LIMIT_BYTES = 60_000_000          # array data of one --dump-outputs directory: under 64 MB with the .npy headers
+
+
+def step_arrays(results, damping):
+    """per unit cell what bp_step_batch returns: the outgoing message of every side, the damped next message (damping only),
+    the message error and the truncation error."""
+    from kagomeperiodicbp_b200.lattice import BLOCK_SIDES_CCW
+    arrays = {}
+    for ci, (out_msgs, next_msgs, err, trunc) in enumerate(results):
+        kinds = [("out", out_msgs)] + ([("next", next_msgs)] if damping else [])
+        for kind, msgs in kinds:
+            for s in BLOCK_SIDES_CCW:
+                for k, t in enumerate(msgs[s].mps.A):
+                    arrays[f"cell{ci}_{kind}_{s}_site{k:02d}"] = t
+        arrays[f"cell{ci}_error"] = np.float64(err)
+        arrays[f"cell{ci}_trunc_error"] = np.float64(trunc)
+    return arrays
+
+
+def write_outputs(path, arrays):
+    """DIR/<name>.npy in float64, complex arrays with a trailing (real, imaginary) axis.  Above DUMP_LIMIT_BYTES every array
+    keeps the same fraction of its elements, flattened, at indices drawn from a fixed seed."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    total = sum(a.size * (16 if np.iscomplexobj(a) else 8) for a in arrays.values())
+    frac = min(1.0, DUMP_LIMIT_BYTES / total)
+    rng = np.random.default_rng(0)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if frac < 1.0 and a.ndim:
+            a = a.reshape(-1)[np.sort(rng.choice(a.size, max(1, int(a.size * frac)), replace=False))]
+        if np.iscomplexobj(a):
+            a = np.stack([a.real, a.imag], axis=-1)
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -293,10 +334,12 @@ def run_reference_arm(a, rank):
     times = []
     for i in range(a.warmup + a.steps):
         t0 = time.perf_counter()
-        obub(T, E, A, SIDE_ANGLE[side], order[:k], D_trunc=chi, ket_tensors=K)
+        mp = obub(T, E, A, SIDE_ANGLE[side], order[:k], D_trunc=chi, ket_tensors=K)
         dt = time.perf_counter() - t0
         if i >= a.warmup:
             times.append(dt)
+    if a.dump_outputs:
+        write_outputs(a.dump_outputs, {f"chain_{side}_site{j:02d}": t for j, t in enumerate(mp.A)})
     sec = float(np.mean(times))
     frac = k / len(order)                 # messages done per step (the early swallows are cheaper than average: favours the CPU)
     v = frac / sec
@@ -356,6 +399,11 @@ class SideSet:
             self.engs[s].sync()
         for s in self.sides:                                       # speculative-graph protocol (include/kbp.h): part of the step
             self.respec += bool(self.comps[s].verify_resident(self.engs[s], (bp.E_SVD_NOCONV,)))
+
+    def collect(self, config):
+        """what the last step left on the engines, per unit cell as bp_step_batch returns it"""
+        res = {s: self.comps[s].collect(self.engs[s], self.B) for s in self.sides}
+        return self.bp.assemble_step(res, self.B, config)
 
     def spec_counters(self):
         out = {"host_driven_reruns": self.respec}
@@ -451,6 +499,7 @@ def main():
     barrier()
     l0, g0, f0 = ss.launches(), ss.graph_counters(), ss.gemm_flops()
     ms_step = timed_steps(ss, a.steps, flush, barrier, torch)
+    last_step = ss.collect(cfg) if a.dump_outputs and rank == 0 else None
     n_launch = ss.launches() - l0
     executed_flops = (ss.gemm_flops() - f0) / a.steps
     g1 = ss.graph_counters()
@@ -480,12 +529,16 @@ def main():
             barrier()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            sh.step()
+            err, trunc, _ = sh.step()
             e1.record()
             torch.cuda.synchronize()
             tot += e0.elapsed_time(e1)
         ms_sharded = tot / a.steps
         gather_bytes = sh.gather_bytes
+        if a.dump_outputs and rank == 0:
+            last_step = [sh.messages() + (err, trunc)]
+    if last_step is not None:
+        write_outputs(a.dump_outputs, step_arrays(last_step, a.damping))
     sampler.stop_flag = True
     sampler.join(timeout=2)
 
