@@ -52,7 +52,12 @@ enum {
   KBP_OP_ZERO = 7,           /* dst, n */
   KBP_OP_SCALAR_TO_SLOT = 8, /* buf, slot_re, slot_im */
   KBP_OP_NONFINITE = 9,      /* buf, n, slot */
-  KBP_OP_EYE = 10            /* dst, rows, cols : dst = identity (reshaped-identity MPS sites, src/libs/bubblecon.py:345-382) */
+  KBP_OP_EYE = 10,           /* dst, rows, cols : dst = identity (reshaped-identity MPS sites, src/libs/bubblecon.py:345-382) */
+  KBP_OP_SU = 11             /* G_A, G_B, G_C, lambda, gate, rdm, d, D, max_steps, tol(bits), slot_steps, slot_delta, slot_nonfinite,
+                                then 6 x (site_i, leg_i, site_j, leg_j):  simple update of the Kagome unit cell (Gamma [d, D, D, D, D]
+                                x 3 and lambda 6 x D updated in place, gate d^4 in the layout g[i', i, j', j], rdm 6 x d^4 written),
+                                one CTA per chain, up to max_steps Trotter steps, a chain stops when its step delta < tol; d = 2,
+                                2 <= D <= 6 */
 };
 
 /* lifetime */

@@ -6,7 +6,7 @@ import subprocess
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
-SOURCES = ["k_util.cu", "k_gemm.cu", "k_qr.cu", "k_qr_cluster.cu", "k_svd.cu", "k_svd_small.cu", "k_tsvd.cu", "kbp_capi.cu"]
+SOURCES = ["k_util.cu", "k_gemm.cu", "k_qr.cu", "k_qr_cluster.cu", "k_svd.cu", "k_svd_small.cu", "k_tsvd.cu", "k_su.cu", "kbp_capi.cu"]
 LIB = os.path.join(HERE, "libkbp.so")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]

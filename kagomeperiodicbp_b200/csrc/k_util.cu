@@ -183,11 +183,13 @@ void init_qr_attributes();
 void init_svd_attributes();
 void init_svd_small_attributes();
 void init_tsvd_attributes();
+void init_su_attributes();
 void init_device_attributes() {
   init_gemm_attributes();
   init_qr_attributes();
   init_svd_attributes();
   init_svd_small_attributes();
   init_tsvd_attributes();
+  init_su_attributes();
 }
 }  // namespace kbp

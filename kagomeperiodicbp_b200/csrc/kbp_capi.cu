@@ -651,6 +651,25 @@ static int run_ops(kbp_ctx* c, const int64_t* w, int64_t n_words, bool capture, 
         i += 4;
         break;
       }
+      case KBP_OP_SU: {
+        NEED(37);
+        const int64_t* v = w + i + 1;
+        const int64_t d = v[6], D = v[7];
+        if (!kbp::su_supported((int)d, (int)D) || v[8] < 0 || !slot_ok(v[10]) || !slot_ok(v[11]) || !slot_ok(v[12])) BAD("su: bad argument");
+        const int64_t elems = d * D * D * D * D, d4 = d * d * d * d;
+        if (!in_arena(v[0], elems) || !in_arena(v[1], elems) || !in_arena(v[2], elems) || !in_arena(v[3], 6 * D) || !in_arena(v[4], d4) ||
+            !in_arena(v[5], 6 * d4))
+          BAD("su: buffer out of arena");
+        int seen[3][4] = {{0}};
+        for (int b = 0; b < 6; ++b)
+          for (int e = 0; e < 2; ++e) {
+            const int64_t s = v[13 + 4 * b + 2 * e], l = v[14 + 4 * b + 2 * e];
+            if (s < 0 || s > 2 || l < 0 || l > 3 || seen[s][l]++) BAD("su: the bond table must pair every virtual leg exactly once");
+          }
+        kbp::simple_update(a, v);
+        i += 38;
+        break;
+      }
       default:
         BAD("unknown opcode");
     }

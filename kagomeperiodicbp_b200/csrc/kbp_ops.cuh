@@ -134,5 +134,8 @@ void eye(const Arena& a, int64_t dst, int64_t rows, int64_t cols);
 void scalar_to_slot(const Arena& a, int64_t buf, int slot_re, int slot_im);
 // NaN/Inf guard: slots[slot] += (number of non-finite entries in buf)
 void count_nonfinite(const Arena& a, int64_t buf, int64_t n, int slot);
+// simple update of the three-site Kagome unit cell, one CTA per chain (k_su.cu); w = the 37 argument words of KBP_OP_SU
+bool su_supported(int d, int D);
+void simple_update(const Arena& a, const int64_t* w);
 
 }  // namespace kbp

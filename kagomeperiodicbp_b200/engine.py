@@ -13,7 +13,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("KBP_LIB") or os.path.join(_HERE, "libkbp.so")      # KBP_LIB: developer override (debug builds)
 
-OP_PERMUTE, OP_GEMM, OP_QR, OP_SVD, OP_NORMALIZE, OP_EMBED, OP_ZERO, OP_SCALAR_TO_SLOT, OP_NONFINITE, OP_EYE = range(1, 11)
+OP_PERMUTE, OP_GEMM, OP_QR, OP_SVD, OP_NORMALIZE, OP_EMBED, OP_ZERO, OP_SCALAR_TO_SLOT, OP_NONFINITE, OP_EYE, OP_SU = range(1, 12)
 E_SVD_NOCONV, E_NONFINITE = -4, -5
 
 EXPORTED = [

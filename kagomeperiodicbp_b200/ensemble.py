@@ -73,15 +73,21 @@ def belief_propagation_batch(N: int, cells: list, config: BPConfig, messages_lis
 
 
 def run_ensemble(seeds, D: int, N: int, chi_factor: float = 1.0, rank: int = 0, world: int = 1, device: int = 0, batch: int = 8,
-                 ite_steps: int = 0, delta_t: float = 1e-2, save_folder: str | None = None, method: int = 3):
+                 ite_steps: int = 0, delta_t: float = 1e-2, save_folder: str | None = None, method: int = 3, init: str = "random"):
     """one row per seed: random unit cell (method 3 of scripts/condor/send_ite.py:66-70) -> batched block BP -> `ite_steps` ITE
-    edge updates per cell -> energy per site.  Returns this rank's rows."""
+    edge updates per cell -> energy per site.  ``init="su"``: the rank's random cells first go through one batched simple
+    update (simple_update.simple_update, default schedule) and BP starts from the SU cells.  Returns this rank's rows."""
+    if init not in ("random", "su"):
+        raise ValueError(f"init must be 'random' or 'su', got {init!r}")
     mine = seeds_of_rank(list(seeds), rank, world)
     chi_bp = int(2 * D * D * chi_factor)
     chi = int((2 * D * D + 10) * chi_factor)
     cfg = BPConfig(trunc_dim=chi_bp, msg_diff_terminate=1e-6, msg_diff_good_enough=1e-5, damping=0.1, max_iterations=50, init_msg="UQ")
     t0 = time.perf_counter()
     cells = [UnitCell.random(2, D, seed=s) for s in mine]
+    if init == "su" and cells:
+        from .simple_update import simple_update
+        cells = [r.unit_cell for r in simple_update(cells, device=device)]
     res = belief_propagation_batch(N, cells, cfg, device=device, batch=batch)
     rows = []
     for s, cell, (msgs, its, err, ok) in zip(mine, cells, res):

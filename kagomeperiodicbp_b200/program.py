@@ -12,8 +12,8 @@ import struct
 
 import numpy as np
 
-from .engine import (OP_EMBED, OP_EYE, OP_GEMM, OP_NONFINITE, OP_NORMALIZE, OP_PERMUTE, OP_QR, OP_SCALAR_TO_SLOT, OP_SVD,
-                     OP_ZERO, qr_work_elems, svd_work_elems)
+from .engine import (OP_EMBED, OP_EYE, OP_GEMM, OP_NONFINITE, OP_NORMALIZE, OP_PERMUTE, OP_QR, OP_SCALAR_TO_SLOT, OP_SU,
+                     OP_SVD, OP_ZERO, qr_work_elems, svd_work_elems)
 
 ALIGN = 8  # complex128 elements (128 B)
 
@@ -274,6 +274,15 @@ class Program:
 
     def nonfinite(self, x: DT, slot: int):
         self._emit(OP_NONFINITE, x.off, x.size, slot)
+
+    def simple_update_(self, gammas, lam: DT, gate: DT, rdm: DT, max_steps: int, tol: float, slots, bonds):
+        """in place: up to ``max_steps`` simple-update steps of the unit cell (Gamma_A, Gamma_B, Gamma_C = ``gammas``, lambda
+        [6, D]) with the two-site gate [d, d, d, d]; writes the six SU-environment RDMs to ``rdm`` [6, d, d, d, d].  ``slots``:
+        (steps done, last step delta, non-finite entries); ``bonds``: six (site_i, leg_i, site_j, leg_j)."""
+        d, D = gammas[0].shape[0], gammas[0].shape[1]
+        (tol_bits,) = struct.unpack("q", struct.pack("d", float(tol)))
+        self._emit(OP_SU, *(t.off for t in gammas), lam.off, gate.off, rdm.off, d, D, int(max_steps), tol_bits, *slots,
+                   *(x for bond in bonds for x in bond))
 
     # ---------------- finish ----------------
     def finalize(self):
