@@ -2,7 +2,7 @@
 //
 // The boundary-MPS chain is a long sequence of SMALL dependent products (m, n of a few hundred at most,
 // k up to a few thousand), so what bounds a product is latency, not the tensor pipe: one CTA computes a
-// BM x BN tile with 8 warps and streams its k-slabs through a 4-stage cp.async ring in shared memory
+// BM x BN tile with 8 warps and streams its k-slabs through a 3- or 4-stage cp.async ring in shared memory
 // (16-byte copies of whole complex128 elements, zero-filled past the edges), one barrier per slab.
 // Tiles are 64x64 (warps 4 x 2, four 16x8 accumulators each) when that already fills the machine, else
 // 32x32 (warps 2 x 4), else 16x16 (2 warps); products with a long k and a tiny output (Gram matrices Y^H Y) can additionally be
@@ -49,6 +49,7 @@ __device__ __forceinline__ unsigned long long gemm_globaltimer() {
 }
 
 constexpr int GEMM_MAX_TILES = 4096;
+constexpr int GEMM_WARPS_TARGET = 900;    // automatic split-K: warps a small product is split up to
 
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem, bool valid) {
   const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
@@ -59,35 +60,7 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
 
-// ---- bulk asynchronous copies (cp.async.bulk, SASS UBLKCP: the TMA unit's 1-D path) completing on an mbarrier
-__device__ __forceinline__ unsigned smem_addr(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_parity(unsigned long long* bar, unsigned parity) {
-  unsigned done = 0;
-  const unsigned a = smem_addr(bar);
-  for (int spins = 0; !done && spins < (1 << 22); ++spins)        // bounded: a lost copy must not hang the GPU
-    asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }" : "=r"(done) : "r"(a), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_copy_g2s(void* smem, const void* gmem, unsigned bytes, unsigned long long* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_addr(smem)), "l"(gmem), "r"(bytes),
-               "r"(smem_addr(bar))
-               : "memory");
-}
-
-// BULK: operand slabs are staged by the TMA unit's bulk copies -- one contiguous tile row (256 B at 16 x 16 tiles) per copy, issued
-// by the lanes of warp 0, completion counted in bytes on one mbarrier per stage -- instead of 16-byte cp.async copies issued by
-// every thread (8 per thread and slab, each with its own address arithmetic).  Only for products whose tiles are all full
-// (m, n multiples of the tile, k of the slab: every product of the D = 4 subspace iteration); others take the cp.async kernel.
-// Opt-in (KBP_GEMM_BULK=1), because it was measured SLOWER on the B200 for these tiles: 512 x 64 x 512 in a program graph 18.4 us
-// against 11.8 us, one D = 4, N = 3 chain 99 against 85 ms -- a 256-byte row per copy is far below what the TMA unit needs to
-// amortise its per-operation cost (~46 cycles of service per copy, shared by the 3-4 CTAs of an SM), and the products are
-// bound by dependent issue, not by the copies.  What would pay is one 2-D tensor-map copy per tile and slab (cp.async.bulk.tensor).
-template <int BM, int BN, int STAGES, int NWARPS, bool A_KC, bool B_KC, bool BULK = false>
+template <int BM, int BN, int STAGES, int NWARPS, bool A_KC, bool B_KC>
 __global__ void __launch_bounds__(32 * NWARPS) zgemm_dmma_kernel(cplx* __restrict__ base, long long chain_stride, GemmArgs g) {
   constexpr int NTHR = 32 * NWARPS;
   constexpr int WMS = BM / 16, WNS = NWARPS / WMS;    // warp grid
@@ -152,34 +125,6 @@ __global__ void __launch_bounds__(32 * NWARPS) zgemm_dmma_kernel(cplx* __restric
     pb[r] = Bb + (b_kc ? (long long)(colok ? col0 + nn : 0) * g.k + (long long)s_begin * BK + kk
                        : ((long long)s_begin * BK + kk) * g.n + (colok ? col0 + nn : 0));
   }
-  __shared__ __align__(8) unsigned long long full_bar[STAGES];
-  if (BULK) {
-    if (t == 0) {
-#pragma unroll
-      for (int s = 0; s < STAGES; ++s) mbar_init(&full_bar[s], 1);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-  }
-  auto issue_bulk = [&](int slab, int stage) {                       // warp 0 only
-    constexpr int rowsA = A_KC ? BM : BK, rowsB = B_KC ? BN : BK;
-    constexpr unsigned bytesA = (A_KC ? BK : BM) * 16u, bytesB = (B_KC ? BK : BN) * 16u;
-    const long long k0 = (long long)(s_begin + slab) * BK;
-    cplx* at = As + stage * TA;
-    cplx* bt = Bs + stage * TB;
-    if (lane == 0) mbar_expect_tx(&full_bar[stage], rowsA * bytesA + rowsB * bytesB);
-    __syncwarp();
-    for (int r = lane; r < rowsA + rowsB; r += 32) {
-      if (r < rowsA) {
-        const cplx* src = A_KC ? Ab + (long long)(row0 + r) * g.k + k0 : Ab + (k0 + r) * g.m + row0;
-        bulk_copy_g2s(at + r * (A_KC ? LDK : LDM), src, bytesA, &full_bar[stage]);
-      } else {
-        const int rb = r - rowsA;
-        const cplx* src = B_KC ? Bb + (long long)(col0 + rb) * g.k + k0 : Bb + (k0 + rb) * g.n + col0;
-        bulk_copy_g2s(bt + rb * (B_KC ? LDK : LDN), src, bytesB, &full_bar[stage]);
-      }
-    }
-  };
   auto issue = [&](int slab, int stage) {
     const int k0 = (s_begin + slab) * BK;
     cplx* at = As + stage * TA;
@@ -211,31 +156,16 @@ __global__ void __launch_bounds__(32 * NWARPS) zgemm_dmma_kernel(cplx* __restric
 #pragma unroll
       for (int j = 0; j < 4; ++j) p1[q4][i][j] = p2[q4][i][j] = p3[q4][i][j] = 0.0;
 
-  if (BULK) {
-    if (w == 0)
-      for (int s = 0; s < STAGES - 1; ++s)
-        if (s < nslab) issue_bulk(s, s);
-  } else {
 #pragma unroll
-    for (int s = 0; s < STAGES - 1; ++s) {
-      if (s < nslab) issue(s, s);
-      cp_async_commit();
-    }
+  for (int s = 0; s < STAGES - 1; ++s) {
+    if (s < nslab) issue(s, s);
+    cp_async_commit();
   }
   for (int slab = 0; slab < nslab; ++slab) {
-    if (BULK) {
-      mbar_wait_parity(&full_bar[slab % STAGES], (unsigned)(slab / STAGES) & 1u);      // the slab has landed
-      __syncthreads();                                 // everyone finished slab-1's stage: it may be refilled
-      if (w == 0 && slab + STAGES - 1 < nslab) {
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy reads of that stage before the async-proxy writes
-        issue_bulk(slab + STAGES - 1, (slab + STAGES - 1) % STAGES);
-      }
-    } else {
-      cp_async_wait<STAGES - 2>();
-      __syncthreads();                                 // slab's data visible; everyone finished slab-1's stage
-      if (slab + STAGES - 1 < nslab) issue(slab + STAGES - 1, (slab + STAGES - 1) % STAGES);
-      cp_async_commit();
-    }
+    cp_async_wait<STAGES - 2>();
+    __syncthreads();                                   // slab's data visible; everyone finished slab-1's stage
+    if (slab + STAGES - 1 < nslab) issue(slab + STAGES - 1, (slab + STAGES - 1) % STAGES);
+    cp_async_commit();
     const cplx* at = As + (slab % STAGES) * TA;
     const cplx* bt = Bs + (slab % STAGES) * TB;
 #pragma unroll
@@ -267,7 +197,7 @@ __global__ void __launch_bounds__(32 * NWARPS) zgemm_dmma_kernel(cplx* __restric
       }
     }
   }
-  if (!BULK) cp_async_wait<0>();
+  cp_async_wait<0>();
   if (g.ktime_slot >= 0 && threadIdx.x == 0) atomicMax(&g_gemm_t1[g.ktime_slot], gemm_globaltimer());   // (epilogue not included)
   if (g.fused) {
     // split-K without a second launch: every CTA parks its partial tile, the last one to arrive at the tile's counter adds
@@ -327,7 +257,7 @@ __global__ void __launch_bounds__(32 * NWARPS) zgemm_dmma_kernel(cplx* __restric
     }
 }
 
-template <int BM, int BN, int STAGES, int NWARPS, bool A_KC, bool B_KC, bool BULK = false>
+template <int BM, int BN, int STAGES, int NWARPS, bool A_KC, bool B_KC>
 static void launch_gemm_l(const Arena& a, GemmArgs g) {
   constexpr int TA = (BM * LDK > BK * (BM + 2)) ? BM * LDK : BK * (BM + 2);
   constexpr int TB = (BN * LDK > BK * (BN + 2)) ? BN * LDK : BK * (BN + 2);
@@ -335,7 +265,7 @@ static void launch_gemm_l(const Arena& a, GemmArgs g) {
   const unsigned tn = (unsigned)((g.n + BN - 1) / BN), tm = (unsigned)((g.m + BM - 1) / BM);
   g.rows_on_x = tm > tn;
   dim3 grid(g.rows_on_x ? tm : tn, g.rows_on_x ? tn : tm, (unsigned)(a.nb * g.ksplit));
-  zgemm_dmma_kernel<BM, BN, STAGES, NWARPS, A_KC, B_KC, BULK><<<grid, 32 * NWARPS, smem, a.stream>>>(a.base, a.chain_stride, g);
+  zgemm_dmma_kernel<BM, BN, STAGES, NWARPS, A_KC, B_KC><<<grid, 32 * NWARPS, smem, a.stream>>>(a.base, a.chain_stride, g);
   ++*a.launches;
 }
 
@@ -344,16 +274,6 @@ static void launch_gemm_l(const Arena& a, GemmArgs g) {
 template <int BM, int BN, int STAGES, int NWARPS>
 static void launch_gemm(const Arena& a, const GemmArgs& g) {
   const bool a_kc = (g.opA == OP_N || g.opA == OP_J), b_kc = (g.opB == OP_T || g.opB == OP_C);
-  if constexpr (BM == 16 && STAGES == 3) {                          // bulk-copy staging: the small-tile kernel, full tiles only
-    static const bool bulk_on = getenv("KBP_GEMM_BULK") != nullptr && atoi(getenv("KBP_GEMM_BULK")) != 0;
-    if (bulk_on && g.m % BM == 0 && g.n % BN == 0 && g.k % BK == 0) {
-      if (a_kc && b_kc) launch_gemm_l<BM, BN, STAGES, NWARPS, true, true, true>(a, g);
-      else if (a_kc) launch_gemm_l<BM, BN, STAGES, NWARPS, true, false, true>(a, g);
-      else if (b_kc) launch_gemm_l<BM, BN, STAGES, NWARPS, false, true, true>(a, g);
-      else launch_gemm_l<BM, BN, STAGES, NWARPS, false, false, true>(a, g);
-      return;
-    }
-  }
   if (a_kc && b_kc) launch_gemm_l<BM, BN, STAGES, NWARPS, true, true>(a, g);
   else if (a_kc) launch_gemm_l<BM, BN, STAGES, NWARPS, true, false>(a, g);
   else if (b_kc) launch_gemm_l<BM, BN, STAGES, NWARPS, false, true>(a, g);
@@ -374,10 +294,8 @@ void gemm_splitk(const Arena& a, int64_t C, int64_t A, int64_t B, int64_t m, int
     const int64_t warps = 2 * tiles16 * a.nb;
     const int64_t slabs = (k + BK - 1) / BK;
     int ks = 1;
-    static const bool no_auto = getenv("KBP_GEMM_NOSPLIT") != nullptr;
-    static const int warps_target = getenv("KBP_GEMM_WARPS_TARGET") ? atoi(getenv("KBP_GEMM_WARPS_TARGET")) : 900;
-    if (!no_auto && warps < 600 && slabs >= 8 && tiles16 <= GEMM_MAX_TILES && a.scratch != nullptr) {
-      ks = (int)((warps_target + warps - 1) / warps);
+    if (warps < 600 && slabs >= 8 && tiles16 <= GEMM_MAX_TILES && a.scratch != nullptr) {
+      ks = (int)((GEMM_WARPS_TARGET + warps - 1) / warps);
       if (ks > slabs / 4) ks = (int)(slabs / 4);
       if (ks > 16) ks = 16;
       while (ks > 1 && (int64_t)ks * m * n > a.scratch_stride) --ks;
@@ -389,21 +307,10 @@ void gemm_splitk(const Arena& a, int64_t C, int64_t A, int64_t B, int64_t m, int
   // few dozen tiles is bound by the handful of SMs it occupies.  Pick the largest tile that still spreads over the machine.
   const int64_t ctas64 = ((n + 63) / 64) * ((m + 63) / 64) * a.nb * g.ksplit;
   const int64_t ctas32 = ((n + 31) / 32) * ((m + 31) / 32) * a.nb * g.ksplit;
-  const int64_t ctas3264 = ((n + 63) / 64) * ((m + 31) / 32) * a.nb * g.ksplit;
-  // opt-in: measured slower on the 8-cell ensemble (six sides 629 against 601 ms per iteration: 128 CTAs of 8 warps leave each SM
-  // sub-partition two warps, too few to cover the fragment-load latency between the DMMAs)
-  static const bool tile3264 = getenv("KBP_GEMM_TILE3264") && atoi(getenv("KBP_GEMM_TILE3264")) != 0;
-  // tuning knobs of the small-product path (tools/gemm_bench.py sweeps them)
-  static const int fused_tile = getenv("KBP_GEMM_FUSED_TILE") ? atoi(getenv("KBP_GEMM_FUSED_TILE")) : 16;
-  static const int stages16 = getenv("KBP_GEMM_STAGES16") ? atoi(getenv("KBP_GEMM_STAGES16")) : 3;   // measured: 3 stages (30 KB, 7 CTAs per SM) beat 4 on every shape of tools/gemm_bench.py d4
-  if (g.fused && fused_tile == 32) launch_gemm<32, 32, 4, 8>(a, g);
-  else if (stages16 == 2 && (g.fused || ctas32 < 96)) launch_gemm<16, 16, 2, 2>(a, g);
-  else if (stages16 == 3 && (g.fused || ctas32 < 96)) launch_gemm<16, 16, 3, 2>(a, g);
-  else if (g.fused) launch_gemm<16, 16, 4, 2>(a, g);
+  // The 16 x 16 tile runs 3 stages: measured, 3 stages (30 KB, 7 CTAs per SM) beat 4 on every shape of tools/gemm_bench.py d4.
+  if (g.fused || ctas32 < 96) launch_gemm<16, 16, 3, 2>(a, g);
   else if (ctas64 >= 96) launch_gemm<64, 64, 3, 8>(a, g);
-  else if (tile3264 && n >= 64 && ctas3264 >= 96) launch_gemm<32, 64, 3, 8>(a, g);   // batched n = b panels (8 chains x 16 row tiles): two
-  else if (ctas32 >= 96) launch_gemm<32, 32, 4, 8>(a, g);                           // 16 x 8 accumulators per warp share every A fragment
-  else launch_gemm<16, 16, 4, 2>(a, g);
+  else launch_gemm<32, 32, 4, 8>(a, g);
 }
 
 template <int BM, int BN, int STAGES, int NWARPS>
@@ -433,11 +340,8 @@ void gemm_ktime_report(const char* tag) {
 }
 
 void init_gemm_attributes() {
-  gemm_attr<16, 16, 4, 2>();
   gemm_attr<16, 16, 3, 2>();
-  gemm_attr<16, 16, 2, 2>();
   gemm_attr<32, 32, 4, 8>();
-  gemm_attr<32, 64, 3, 8>();
   gemm_attr<64, 64, 3, 8>();
 }
 

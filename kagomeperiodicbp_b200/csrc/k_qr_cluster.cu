@@ -17,7 +17,6 @@
 
 #include <cooperative_groups.h>
 #include <math.h>
-#include <stdlib.h>
 
 namespace cg = cooperative_groups;
 
@@ -261,24 +260,23 @@ size_t qrc_smem(int m, int n, int C) {
   return sizeof(double2) * (size_t)(n + kk) * ld + sizeof(double) * ((size_t)2 * C * NV + 2 * NV + ((kk + 1) & ~1) + 4 * 16 + 2) + 64;
 }
 
+// smallest cluster (1, 2, 4 or 8 CTAs) whose row slices and shared memory fit, 0 if the shape is not handled here
+int qrc_cluster_size(int64_t m, int64_t n) {
+  if (m > 8 * QRC_MLOC_MAX || n > 256) return 0;
+  int C = 1;
+  while (C <= 8 && ((m + C - 1) / C > QRC_MLOC_MAX || qrc_smem((int)m, (int)n, C) > QRC_SMEM_MAX)) C <<= 1;
+  return C <= 8 ? C : 0;
+}
+
 }  // namespace
 
 // does the cluster kernel take this shape?
-bool qr_cluster_fits(int64_t m, int64_t n) {
-  static const bool on = !(getenv("KBP_QR_CLUSTER") && atoi(getenv("KBP_QR_CLUSTER")) == 0);
-  if (!on || m > 8 * QRC_MLOC_MAX || n > 256) return false;
-  int C = 1;
-  while (C <= 8 && ((m + C - 1) / C > QRC_MLOC_MAX || qrc_smem((int)m, (int)n, C) > QRC_SMEM_MAX)) C <<= 1;
-  return C <= 8;
-}
+bool qr_cluster_fits(int64_t m, int64_t n) { return qrc_cluster_size(m, n) > 0; }
 
 // returns false if the shape is not handled here (caller uses the one-CTA kernel)
 bool qr_cluster(const Arena& a, int64_t A, int64_t Q, int64_t R, int64_t m, int64_t n) {
-  static const bool on = !(getenv("KBP_QR_CLUSTER") && atoi(getenv("KBP_QR_CLUSTER")) == 0);
-  if (!on || m > 8 * QRC_MLOC_MAX || n > 256) return false;
-  int C = 1;
-  while (C <= 8 && ((m + C - 1) / C > QRC_MLOC_MAX || qrc_smem((int)m, (int)n, C) > QRC_SMEM_MAX)) C <<= 1;
-  if (C > 8) return false;
+  const int C = qrc_cluster_size(m, n);
+  if (C == 0) return false;
   QrcArgs g;
   g.A = A; g.Q = Q; g.R = R; g.m = (int)m; g.n = (int)n; g.mask = a.mask; g.mask_want = a.mask_want;
   cudaLaunchConfig_t cfg = {};

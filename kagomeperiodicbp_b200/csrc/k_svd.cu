@@ -31,6 +31,7 @@ constexpr int LDP = KC + 4;   // shared row stride (doubles): 36 mod 16 == 4 -> 
 constexpr size_t SVD_ROUND_SMEM = 3 * sizeof(double2) * PR * (PR + 1) + 2 * sizeof(double) * PR * LDP;
 constexpr double SVD_TOL = 1e-14;
 constexpr int SVD_MAX_SWEEPS = 40;
+constexpr int SVD_INNER_LO = 2;          // inner Jacobi sweeps of a block pair during the first 24 outer sweeps (15 after)
 
 static inline int64_t round_up(int64_t x, int64_t a) { return (x + a - 1) / a * a; }
 
@@ -473,11 +474,10 @@ __global__ void svd_exact_sweep_end_kernel(SvdCtl* __restrict__ ctl, double* __r
   if (use_handle) cudaGraphSetConditional(h_sweep, any ? 1u : 0u);
 }
 
-static void svd_exact_sweep(const Arena& a, int64_t work, const SvdGeom& g, double* prev, double* cur, double* fro2, int inner_lo,
-                            cudaGraphConditionalHandle h_sweep) {
+static void svd_exact_sweep(const Arena& a, int64_t work, const SvdGeom& g, double* prev, double* cur, double* fro2, cudaGraphConditionalHandle h_sweep) {
   cudaMemsetAsync(cur, 0, sizeof(double) * a.nb, a.stream);
   for (int r = 0; r < g.nblk - 1; ++r) {
-    svd_round_kernel<<<dim3(g.nblk / 2, a.nb), 256, SVD_ROUND_SMEM, a.stream>>>(a.base, a.chain_stride, work, g, r, SVD_TOL, prev, cur, fro2, inner_lo, a.ctl);
+    svd_round_kernel<<<dim3(g.nblk / 2, a.nb), 256, SVD_ROUND_SMEM, a.stream>>>(a.base, a.chain_stride, work, g, r, SVD_TOL, prev, cur, fro2, SVD_INNER_LO, a.ctl);
     ++*a.launches;
   }
   svd_exact_sweep_end_kernel<<<1, 32, 0, a.stream>>>(a.ctl, prev, cur, a.nb, SVD_TOL, SVD_MAX_SWEEPS, a.slots, a.n_slots, h_sweep, a.capture ? 1 : 0);
@@ -489,7 +489,6 @@ static void svd_exact_sweep(const Arena& a, int64_t work, const SvdGeom& g, doub
 int svd_exact(const Arena& a, int64_t A, int64_t US, int64_t Vh, int64_t work, int64_t m, int64_t n, int64_t keep, int nr_bulk,
               int slot_lognorm, int slot_trunc) {
   static const bool debug = getenv("KBP_SVD_DEBUG") != nullptr;
-  static const int inner_lo = getenv("KBP_SVD_INNER") ? atoi(getenv("KBP_SVD_INNER")) : 2;
   if (debug) fprintf(stderr, "[kbp svd %lldx%lld keep %lld] block-Jacobi path\n", (long long)m, (long long)n, (long long)keep);
   SvdGeom g = svd_geom(m, n);
   {
@@ -513,12 +512,12 @@ int svd_exact(const Arena& a, int64_t A, int64_t US, int64_t Vh, int64_t work, i
   if (a.capture) {
     Arena body;
     if (!begin_cond_body(a, h_sweep, true, &body)) return -1;
-    svd_exact_sweep(body, work, g, prev, cur, fro2, inner_lo, h_sweep);
+    svd_exact_sweep(body, work, g, prev, cur, fro2, h_sweep);
     if (!end_body(body)) return -1;
   } else {
     sweeps = 0;
     while (true) {
-      svd_exact_sweep(a, work, g, prev, cur, fro2, inner_lo, h_sweep);
+      svd_exact_sweep(a, work, g, prev, cur, fro2, h_sweep);
       ++sweeps;
       cudaMemcpyAsync(a.ctl_host, a.ctl, sizeof(SvdCtl), cudaMemcpyDeviceToHost, a.stream);
       if (stream_wait(a) != cudaSuccess) return -1;
@@ -573,22 +572,19 @@ bool svd_reducible(int64_t m, int64_t n) {
 int svd_truncate(const Arena& a, int64_t A, int64_t US, int64_t Vh, int64_t work, int64_t m, int64_t n, int64_t keep,
                  int nr_bulk, int slot_lognorm, int slot_trunc) {
   if (m == 0 || n == 0) return 0;
-  static const int force = getenv("KBP_SVD_FORCE") ? atoi(getenv("KBP_SVD_FORCE")) : 0;   // 1: block-Jacobi only, 2: no small kernel
-  if (force != 1) {
-    if (force != 2 && svd_small_fits(m, n)) {
-      svd_small(a, A, n, US, Vh, m, n, keep, nr_bulk, slot_lognorm, slot_trunc);
-      phase_fix(a, Vh, US, m, n, keep, 1);
-      ++a.counters[1];
-      return 1;
-    }
-    if (force != 2 && svd_reducible(m, n)) {
-      svd_reduced(a, A, US, Vh, work, m, n, keep, nr_bulk, slot_lognorm, slot_trunc);
-      ++a.counters[0];
-      return 1;
-    }
-    const int b = tsvd_block(m, n, keep);
-    if (b > 0) return svd_truncate_subspace(a, A, US, Vh, work, m, n, keep, nr_bulk, slot_lognorm, slot_trunc, b);
+  if (svd_small_fits(m, n)) {
+    svd_small(a, A, n, US, Vh, m, n, keep, nr_bulk, slot_lognorm, slot_trunc);
+    phase_fix(a, Vh, US, m, n, keep, 1);
+    ++a.counters[1];
+    return 1;
   }
+  if (svd_reducible(m, n)) {
+    svd_reduced(a, A, US, Vh, work, m, n, keep, nr_bulk, slot_lognorm, slot_trunc);
+    ++a.counters[0];
+    return 1;
+  }
+  const int b = tsvd_block(m, n, keep);
+  if (b > 0) return svd_truncate_subspace(a, A, US, Vh, work, m, n, keep, nr_bulk, slot_lognorm, slot_trunc, b);
   Arena all = a;
   all.mask = nullptr;
   return svd_exact(all, A, US, Vh, work, m, n, keep, nr_bulk, slot_lognorm, slot_trunc);

@@ -23,7 +23,6 @@
 #include <cooperative_groups.h>
 #include <math.h>
 #include <stdio.h>
-#include <stdlib.h>
 
 namespace cg = cooperative_groups;
 
@@ -230,6 +229,7 @@ __global__ void __launch_bounds__(CACHED ? 768 : 1024) svd_small_kernel(cplx* __
 // recomputed everywhere.  The price is one cluster barrier (~400 cycles) + 32 B x pairs x C of DSMEM traffic per step.
 constexpr int CL_C = 4;     // CTAs per cluster
 constexpr int CL_G = 8;     // lanes per row pair
+constexpr int CL_MIN_P = 48; // smallest p that takes the cluster kernel
 
 // The per-step exchange does not use the cluster barrier (its release fence costs ~900 cycles per step here): partial sums
 // travel as asynchronous DSMEM stores that complete a transaction count on the RECEIVER's mbarrier (st.async ...
@@ -508,10 +508,7 @@ void svd_small(const Arena& a, int64_t A, int64_t lda, int64_t US, int64_t Vh, i
   g.nr_bulk = nr_bulk; g.slot_lognorm = slot_lognorm; g.slot_trunc = slot_trunc;
   const int p = (int)(m < n ? m : n), pp = (p + 1) & ~1, npairs = pp / 2 > 0 ? pp / 2 : 1;
   const int q = (int)(m <= n ? n : m + n);
-  // cluster version for the larger matrices (KBP_SMALL_CLUSTER=0: off; KBP_SMALL_CLUSTER_MINP = smallest p that uses it)
-  static const bool cluster_on = !(getenv("KBP_SMALL_CLUSTER") && atoi(getenv("KBP_SMALL_CLUSTER")) == 0);
-  static const int cluster_minp = getenv("KBP_SMALL_CLUSTER_MINP") ? atoi(getenv("KBP_SMALL_CLUSTER_MINP")) : 48;
-  if (cluster_on && p >= cluster_minp) {
+  if (p >= CL_MIN_P) {                              // cluster version for the larger matrices
     // (4 and 2 lanes per pair were measured slower: the per-lane FP64 work grows faster than the shuffles shrink)
     const int C = CL_C, ql = (q + C - 1) / C, Gc = CL_G;
     const int cpl = (ql + Gc - 1) / Gc;

@@ -18,7 +18,6 @@
 #include "kbp_common.cuh"
 #include "kbp_ops.cuh"
 
-#include <cooperative_groups.h>
 #include <mutex>
 #include <vector>
 
@@ -87,13 +86,14 @@ constexpr double TSVD_MIN_RATIO = 1e-6;
 
 static inline int64_t rup8(int64_t x) { return (x + 7) / 8 * 8; }
 
+// block = 2.0 x keep.  Measured on the D=4, N=3 side program (B200, whole program as one graph, profiles/r02_SUMMARY.md):
+// 1.5 -> 136 ms, 1.7 -> 122, 2.0 -> 112.5, 2.2 -> 132, 2.5 -> 133, 3.0 -> 151 per chain: a wider block saves iterations
+// (8.0 at 2.5 vs 9.6 at 2.0 on average) but every b x b kernel of an iteration (Cholesky, Jacobi, triangular solve) gets slower
+constexpr int TSVD_BLOCK_FACTOR = 2;
+
 int tsvd_block(int64_t m, int64_t n, int64_t keep) {
-  // block = 2.0 x keep.  Measured on the D=4, N=3 side program (B200, whole program as one graph, profiles/r02_SUMMARY.md):
-  // 1.5 -> 136 ms, 1.7 -> 122, 2.0 -> 112.5, 2.2 -> 132, 2.5 -> 133, 3.0 -> 151 per chain: a wider block saves iterations
-  // (8.0 at 2.5 vs 9.6 at 2.0 on average) but every b x b kernel of an iteration (Cholesky, Jacobi, triangular solve) gets slower
-  static const int factor_x10 = getenv("KBP_TSVD_FACTOR_X10") ? atoi(getenv("KBP_TSVD_FACTOR_X10")) : 20;
   const int64_t p = m < n ? m : n;
-  int64_t b = rup8(keep * factor_x10 / 10);
+  int64_t b = rup8(TSVD_BLOCK_FACTOR * keep);
   if (b > TSVD_BMAX2) b = TSVD_BMAX2;
   if (b < keep + 8 || b * 100 > p * 80) return 0;     // not worth it / not applicable
   return (int)b;
@@ -437,28 +437,6 @@ __device__ __forceinline__ void chol_reg_from_partials(const CholWork& w, const 
   chol_factor_reg<NC>(w, b, t, v);
 }
 
-// the same from a Gram matrix already in w.S (R overwrites it)
-template <int NC>
-__device__ __forceinline__ void chol_reg_from_smem(const CholWork& w, int b, int t) {
-  constexpr int NR = 2 * NC;
-  const int lane = t & 31, wp = t >> 5;
-  cplx v[NR][NC];
-#pragma unroll
-  for (int r = 0; r < NR; ++r)
-#pragma unroll
-    for (int k = 0; k < NC; ++k) {
-      v[r][k] = cmake(0.0, 0.0);
-      if (2 * k + 1 >= r) {
-        const int i = wp + 16 * r, c = lane + 32 * k;
-        if (i < b && c < b && c >= i) {
-          v[r][k] = w.S[i * w.ld + c];
-          if (c == i) w.diag0[i] = v[r][k].x;
-        }
-      }
-    }
-  chol_factor_reg<NC>(w, b, t, v);
-}
-
 constexpr int CREG_BMAX = 96;             // widest matrix of the register-resident factorisation (NC = 3: 12 entries per thread)
 
 // One kernel per register-block count NC (and one for the blocked fallback), so that each gets its own register
@@ -583,195 +561,6 @@ static void launch_chol(const Arena& a, int64_t Gp, int split, int64_t R_out, in
   else if (b <= CREG_BMAX) chol_reg_kernel<3><<<a.nb, 512, smem, a.stream>>>(a.base, a.chain_stride, g, stat);
   else chol_blocked_kernel<<<a.nb, 512, smem, a.stream>>>(a.base, a.chain_stride, g, stat);
   ++*a.launches;
-}
-
-// ------------------------------------------------------------------------------------------------
-// Cholesky-QR of a tall panel in ONE launch:  Out (rows x b) = Y R^{-1},  Y^H Y = R^H R.
-// A cluster of C CTAs splits the rows (RL = 32 or 64 each); every CTA
-//   1. loads its slab into shared memory and forms the partial Gram matrix of it (upper triangle),
-//   2. takes part in an all-reduce over distributed shared memory: CTA k sums slice k of all partials in rank order (every
-//      CTA ends up with bitwise the same matrix) and stores the sums into every CTA's copy,
-//   3. runs the Cholesky factorisation redundantly (same code as chol_kernel: the factorisation is latency bound, not
-//      work bound, and this way R never leaves the SM),
-//   4. solves its slab against R in place (blocked forward substitution with the inverses of the diagonal blocks).
-// Replaces split-K Gram GEMM + chol_kernel + trsm_kernel (three launches, R and the Gram partials through L2).
-// out_rows == 0: only R is wanted.  Rank 0 writes R and the pivot statistic.
-namespace cgx = cooperative_groups;
-
-struct CholQrArgs {
-  long long Y, Out, R;     // arena offsets; Out < 0: R only; R < 0: R not stored
-  int rows, b, rl;         // rl = rows per CTA
-  const int* mask;
-  int mask_want;
-};
-
-__global__ void __launch_bounds__(512) cholqr_cluster_kernel(cplx* __restrict__ base, long long chain_stride, CholQrArgs g, double* __restrict__ stat) {
-  if (g.mask && g.mask[blockIdx.y] != g.mask_want) return;
-  cgx::cluster_group cluster = cgx::this_cluster();
-  const int rank = (int)cluster.block_rank(), C = (int)cluster.num_blocks();
-  extern __shared__ __align__(16) unsigned char cq_raw[];
-  __shared__ cplx rowbuf[4 * CREG_LINE];
-  const int b = g.b, ld = b + 1, rl = g.rl, nblk = (b + CNB - 1) / CNB;
-  CholWork w;
-  w.ld = ld;
-  w.S = reinterpret_cast<cplx*>(cq_raw);                           // b x ld
-  cplx* Ys = w.S + (size_t)b * ld;                                 // rl x ld: the CTA's slab, solved in place
-  cplx* Xs = Ys + (size_t)rl * ld;                                 // nblk x 16 x 16
-  cplx* tmp = Xs + (size_t)nblk * CNB * CNB;                       // 32 x 17
-  w.diag0 = reinterpret_cast<double*>(tmp + 32 * 17);
-  w.dinv = w.diag0 + b;
-  w.piv = w.dinv + b;
-  w.rowbuf = rowbuf;
-  cplx* S = w.S;
-  cplx* cb = base + (long long)blockIdx.y * chain_stride;
-  const int t = threadIdx.x, nt = blockDim.x, lane = t & 31, wp = t >> 5, nw = nt >> 5;
-  const int r0 = rank * rl;
-  // ---- 1. slab
-  {
-    const cplx* Y = cb + g.Y;
-    for (int r = wp; r < rl; r += nw) {
-      const bool ok = r0 + r < g.rows;
-      for (int c = lane; c < b; c += 32) Ys[r * ld + c] = ok ? Y[(long long)(r0 + r) * b + c] : cmake(0.0, 0.0);
-    }
-  }
-  __syncthreads();
-  // partial Gram, upper triangle: thread -> 2 x 2 block (i, i + 1) x (j, j + 1) of the b x b matrix, rows of the slab streamed
-  {
-    const int hb = (b + 1) / 2;
-    for (int e = t; e < hb * hb; e += nt) {
-      const int bi = e / hb, bj = e - bi * hb;
-      if (bj < bi) continue;
-      const int i = 2 * bi, j = 2 * bj;
-      const bool i1 = i + 1 < b, j1 = j + 1 < b;
-      cplx a00 = cmake(0.0, 0.0), a01 = a00, a10 = a00, a11 = a00;
-      for (int r = 0; r < rl; ++r) {
-        const cplx yi = Ys[r * ld + i], yj = Ys[r * ld + j];
-        const cplx yi1 = i1 ? Ys[r * ld + i + 1] : cmake(0.0, 0.0), yj1 = j1 ? Ys[r * ld + j + 1] : cmake(0.0, 0.0);
-        a00 = cadd(a00, ccmul(yi, yj));
-        a01 = cadd(a01, ccmul(yi, yj1));
-        a10 = cadd(a10, ccmul(yi1, yj));
-        a11 = cadd(a11, ccmul(yi1, yj1));
-      }
-      S[i * ld + j] = a00;
-      if (j1) S[i * ld + j + 1] = a01;
-      if (i1) S[(i + 1) * ld + j] = a10;                           // (below the diagonal when bi == bj: never read)
-      if (i1 && j1) S[(i + 1) * ld + j + 1] = a11;
-    }
-  }
-  // ---- 2. all-reduce over the cluster (rank order: deterministic and identical everywhere)
-  if (C > 1) {
-    cluster.sync();
-    const int total = b * ld;
-    const int per = (total + C - 1) / C, e0 = rank * per, e1 = min(total, e0 + per);
-    cplx acc[4];                                                   // host guarantees per <= 4 * blockDim
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const int e = e0 + t + k * nt;
-      const int r = e / ld, c = e - r * ld;
-      cplx v = cmake(0.0, 0.0);
-      if (e < e1 && c >= r && c < b) {                             // upper triangle only
-        for (int q = 0; q < C; ++q) v = cadd(v, cluster.map_shared_rank(S, q)[e]);
-      }
-      acc[k] = v;
-    }
-    cluster.sync();                                                // every partial has been read
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const int e = e0 + t + k * nt;
-      const int r = e / ld, c = e - r * ld;
-      if (e < e1 && c >= r && c < b) {
-        for (int q = 0; q < C; ++q) cluster.map_shared_rank(S, q)[e] = acc[k];
-      }
-    }
-    cluster.sync();
-  } else {
-    __syncthreads();
-  }
-  // ---- 3. Cholesky (redundant per CTA)
-  if (b <= 32) chol_reg_from_smem<1>(w, b, t);
-  else if (b <= 64) chol_reg_from_smem<2>(w, b, t);
-  else if (b <= CREG_BMAX) chol_reg_from_smem<3>(w, b, t);
-  else {
-    for (int i = t; i < b; i += nt) w.diag0[i] = S[i * ld + i].x;
-    __syncthreads();
-    chol_factor(w, b, t, nt);
-  }
-  if (rank == 0) {
-    if (g.R >= 0) {
-      cplx* R = cb + g.R;
-      for (int r = wp; r < b; r += nw)
-        for (int c = lane; c < b; c += 32) R[(long long)r * b + c] = c >= r ? S[r * ld + c] : cmake(0.0, 0.0);
-    }
-    if (t < 32) {
-      const double mn = chol_min_pivot(w, b, t);
-      if (t == 0) stat[blockIdx.y] = fmin(stat[blockIdx.y], mn);
-    }
-  }
-  if (g.Out < 0) return;
-  chol_diag_inverses(w, b, Xs, t, nt);
-  __syncthreads();
-  // ---- 4. slab <- slab R^{-1}: 32 rows per pass, 16 threads per row (half warp), panel by panel
-  for (int pass = 0; pass < rl; pass += 32) {
-    const int r = pass + (t >> 4), c = t & 15;
-    cplx* xr = Ys + r * ld;
-    cplx* tr = tmp + (t >> 4) * 17;
-    for (int pb = 0; pb < nblk; ++pb) {
-      const int p0 = pb * CNB, col = p0 + c;
-      cplx acc = col < b ? xr[col] : cmake(0.0, 0.0);
-      {
-        cplx acc2 = cmake(0.0, 0.0);
-        int i = 0;
-        for (; i + 1 < p0; i += 2) {                                 // two independent chains; R[i][col] from the factor in S
-          const cplx v0 = cmul(xr[i], col < b ? S[i * ld + col] : cmake(0.0, 0.0));
-          const cplx v1 = cmul(xr[i + 1], col < b ? S[(i + 1) * ld + col] : cmake(0.0, 0.0));
-          acc.x -= v0.x; acc.y -= v0.y;
-          acc2.x -= v1.x; acc2.y -= v1.y;
-        }
-        acc.x += acc2.x; acc.y += acc2.y;
-      }
-      tr[c] = acc;
-      __syncwarp();
-      cplx x = cmake(0.0, 0.0);
-      const cplx* X = Xs + pb * CNB * CNB;
-#pragma unroll
-      for (int cp = 0; cp < CNB; ++cp)
-        if (cp <= c) x = cfma(tr[cp], X[cp * CNB + c], x);
-      __syncwarp();
-      if (col < b) xr[col] = x;
-      __syncwarp();
-    }
-  }
-  __syncthreads();
-  {
-    cplx* Out = cb + g.Out;
-    for (int r = wp; r < rl; r += nw) {
-      if (r0 + r >= g.rows) break;
-      for (int c = lane; c < b; c += 32) Out[(long long)(r0 + r) * b + c] = Ys[r * ld + c];
-    }
-  }
-}
-
-static size_t cholqr_cluster_smem(int b, int rl) {
-  const int ld = b + 1, nblk = (b + CNB - 1) / CNB;
-  return sizeof(double2) * ((size_t)b * ld + (size_t)rl * ld + (size_t)nblk * CNB * CNB + 32 * 17) + 3 * sizeof(double) * (size_t)b + 64;
-}
-
-// rows per CTA (0: shape not handled by the cluster kernel)
-static int cholqr_cluster_rl(int64_t rows, int b) {
-  // opt-in (KBP_CHOLQR_CLUSTER=1): one launch instead of three, but measured SLOWER on the B200 (118 us against 17 + 56 + 21 us at
-  // b = 80: the slab Gram and the in-place solve are bound by the shared-memory pipe of the 8 SMs a cluster has, where the
-  // split-K Gram GEMM and the 16-CTA solve spread over the chip); kept for the DMMA version of its Gram stage
-  static const bool on = getenv("KBP_CHOLQR_CLUSTER") && atoi(getenv("KBP_CHOLQR_CLUSTER")) != 0;
-  if (!on) return 0;
-  for (int rl = 64; rl >= 32; rl >>= 1) {
-    if ((rows + rl - 1) / rl > 8) continue;
-    if (cholqr_cluster_smem(b, rl) > 217 * 1024) continue;
-    // the all-reduce keeps at most 4 entries per thread in registers
-    const int C = (int)((rows + rl - 1) / rl);
-    if (((int64_t)b * (b + 1) + C - 1) / C > 4 * 512) continue;
-    return rl;
-  }
-  return 0;
 }
 
 // Out (rows x b) = Y R^{-1} for upper-triangular R by block forward substitution over the 16-column panels:
@@ -1066,35 +855,6 @@ static inline int grid1d(long long n) {
 constexpr int GRAM_SPLIT = 4;
 
 static int64_t cholqr_pass_narrow(const Arena& a, int64_t Y, int64_t T, int64_t Gp, int64_t Dinv, int64_t R_out, int64_t rows, int b, double* stat) {
-  if (const int rl = cholqr_cluster_rl(rows, b)) {
-    CholQrArgs g{Y, T, R_out, (int)rows, b, rl, a.mask, a.mask_want};
-    const int C = (int)((rows + rl - 1) / rl);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)C, (unsigned)a.nb);
-    cfg.blockDim = dim3(512);
-    cfg.dynamicSmemBytes = cholqr_cluster_smem(b, rl);
-    cfg.stream = a.stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = (unsigned)C;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    const cudaError_t le = cudaLaunchKernelEx(&cfg, cholqr_cluster_kernel, a.base, (long long)a.chain_stride, g, stat);
-    if (le == cudaSuccess) {
-      ++*a.launches;
-      PM(2);
-      return T;
-    }
-    static bool warned = false;
-    if (!warned) {
-      warned = true;
-      fprintf(stderr, "[kbp] cholqr_cluster_kernel launch refused (%s; rows %lld b %d cluster %d smem %zu): three-kernel path\n", cudaGetErrorString(le),
-              (long long)rows, b, C, (size_t)cfg.dynamicSmemBytes);
-    }
-    cudaGetLastError();                         // cluster launch refused: three-kernel path
-  }
   const int split = rows >= 256 ? GRAM_SPLIT : 1;
   gemm_splitk(a, Gp, Y, Y, b, b, rows, OP_C, OP_N, split);
   PM(1);
@@ -1344,8 +1104,20 @@ static void tsvd_more_round(const Arena& a, const TsvdBufs& w, int64_t A, int64_
   ++*a.launches;
 }
 
+// Iterations of round 1 from the pseudo-random block (the spectra of the Kagome block need 4-8 for a 1e-13 residual, see the top).
+constexpr int TSVD_IT_COLD = 7;
+// cold start: after TSVD_SAFE_ITERS SAFE iterations the block is already ordered well enough (contamination of column j by a
+// larger direction i has decayed as (s_j/s_i)^(2k), one fast step amplifies it by (s_i/s_j)^2) for the FAST form
+constexpr int TSVD_SAFE_ITERS = 2;
+// SPECULATIVE capture (Arena::speculate): an op whose host-driven run was settled by the subspace iteration within four
+// rounds gets that schedule plus TSVD_SPEC_SLACK iterations and NO conditional node -- a conditional node makes the GPU drain
+// every kernel in flight, also those of the other program graphs running beside this one (six side programs: each of the
+// ~550 nodes per chain waited for some other chain's 300 us Jacobi kernel).  The acceptance test still runs; a miss
+// raises SvdCtl::spec_fail and the host reruns the program host-driven, which also re-learns the schedule.
+constexpr int TSVD_SPEC_SLACK = 1;
+
 // Two kinds of iteration.  SAFE (cold start, Q arbitrary): W = A Q, Y = orth(W), Z = A^H Y, Q = orth(Z).  FAST (Q holds
-// approximate Ritz vectors in decreasing order -- after `safe0` SAFE iterations of a cold start, or after a Rayleigh-Ritz
+// approximate Ritz vectors in decreasing order -- after TSVD_SAFE_ITERS SAFE iterations of a cold start, or after a Rayleigh-Ritz
 // step): the columns of A Q and of A^H A Q are then nearly orthogonal, their Gram matrices are diagonally dominant after
 // scaling, and ONE Cholesky-QR of Z = A^H (A Q) per iteration is as accurate as the safe sequence (the Cholesky kernel
 // reports its smallest pivot / diagonal; a round built on a pivot ratio below TSVD_PIVOT_TRUST is not accepted).
@@ -1356,32 +1128,20 @@ static void tsvd_more_round(const Arena& a, const TsvdBufs& w, int64_t A, int64_
 int svd_truncate_subspace(const Arena& a0, int64_t A, int64_t US, int64_t Vh, int64_t work, int64_t m, int64_t n, int64_t keep,
                           int nr_bulk, int slot_lognorm, int slot_trunc, int b) {
   static const bool debug = getenv("KBP_SVD_DEBUG") != nullptr;
-  static const int it_default = getenv("KBP_TSVD_IT0") ? atoi(getenv("KBP_TSVD_IT0")) : 7;
-  static const bool learn = !(getenv("KBP_TSVD_LEARN") && atoi(getenv("KBP_TSVD_LEARN")) == 0);
   // An op that needed r > 1 rounds when its program ran host-driven (previous BP iteration: nearly the same spectrum) gets
   // the iterations of those rounds up front in the captured graph: one Rayleigh-Ritz step + check instead of r.
-  int it_cold = it_default;
-  // SPECULATIVE capture (Arena::speculate): an op whose host-driven run was settled by the subspace iteration within four
-  // rounds gets that schedule plus `spec_slack` iterations and NO conditional node -- a conditional node makes the GPU drain
-  // every kernel in flight, also those of the other program graphs running beside this one (six side programs: each of the
-  // ~550 nodes per chain waited for some other chain's 300 us Jacobi kernel).  The acceptance test still runs; a miss
-  // raises SvdCtl::spec_fail and the host reruns the program host-driven, which also re-learns the schedule.
-  static const int spec_slack = getenv("KBP_TSVD_SPEC_SLACK") ? atoi(getenv("KBP_TSVD_SPEC_SLACK")) : 1;
+  int it_cold = TSVD_IT_COLD;
   bool spec = false;
-  if (learn && a0.capture && a0.tsvd_rounds) {
+  if (a0.capture && a0.tsvd_rounds) {
     auto f = a0.tsvd_rounds->find(a0.op_key);
-    if (f != a0.tsvd_rounds->end() && f->second > 1) it_cold = it_default + ((f->second < 4 ? f->second : 4) - 1) * TSVD_IT_MORE;
+    if (f != a0.tsvd_rounds->end() && f->second > 1) it_cold = TSVD_IT_COLD + ((f->second < 4 ? f->second : 4) - 1) * TSVD_IT_MORE;
     if (a0.speculate && f != a0.tsvd_rounds->end() && f->second >= 1 && f->second <= 4) {
       spec = true;
-      it_cold += spec_slack;
+      it_cold += TSVD_SPEC_SLACK;
     }
   }
-  // cold start: after `safe0` SAFE iterations the block is already ordered well enough (contamination of column j by a
-  // larger direction i has decayed as (s_j/s_i)^(2k), one fast step amplifies it by (s_i/s_j)^2) for the FAST form
-  static const int safe0 = getenv("KBP_TSVD_SAFE0") ? atoi(getenv("KBP_TSVD_SAFE0")) : 2;
   // a block narrower than 2.5 keep converges more slowly: more iterations are still far cheaper than the exact path
-  static const int it_max_env = getenv("KBP_TSVD_ITMAX") ? atoi(getenv("KBP_TSVD_ITMAX")) : 0;
-  const int it_max = it_max_env > 0 ? it_max_env : (2 * b >= 5 * keep ? 24 : 72);
+  const int it_max = 2 * b >= 5 * keep ? 24 : 72;
   const int max_rounds = 1 + (it_max > it_cold ? (it_max - it_cold + TSVD_IT_MORE - 1) / TSVD_IT_MORE : 0);
   if (keep > 128) return svd_exact(a0, A, US, Vh, work, m, n, keep, nr_bulk, slot_lognorm, slot_trunc);
   Arena a = a0;
@@ -1424,7 +1184,7 @@ int svd_truncate_subspace(const Arena& a0, int64_t A, int64_t US, int64_t Vh, in
   for (int done = 0; done < it_cold; ++done) {
     gemm(a, f0, A, Qb, m, b, n, OP_N, OP_N);                          // W = A Q          -> f0
     PM(0);
-    if (done >= safe0) {
+    if (done >= TSVD_SAFE_ITERS) {
       if (!cold_fast) {                                               // pivots of the SAFE start say nothing about the FAST steps
         tsvd_fill_kernel<<<(a.nb + 127) / 128, 128, 0, a.stream>>>(stat, a.nb, 1.0);
         ++*a.launches;
@@ -1509,8 +1269,7 @@ int svd_truncate_subspace(const Arena& a0, int64_t A, int64_t US, int64_t Vh, in
 void qr_householder(const Arena& a, int64_t A, int64_t Q, int64_t R, int64_t work, int64_t m, int64_t n);   // k_qr.cu
 
 bool qr_cholqr2(const Arena& a0, int64_t A, int64_t Q, int64_t R, int64_t work, int64_t m, int64_t n) {
-  static const bool on = !(getenv("KBP_QR_CHOLQR2") && atoi(getenv("KBP_QR_CHOLQR2")) == 0);
-  if (!on || a0.mask != nullptr || n < 8 || n > CREG_BMAX || m < 4 * n) return false;
+  if (a0.mask != nullptr || n < 8 || n > CREG_BMAX || m < 4 * n) return false;
   const int b = (int)n, nblk = (b + CNB - 1) / CNB;
   const int64_t bb = n * n, need = m * n + GRAM_SPLIT * bb + 2 * bb + n + (int64_t)nblk * CNB * CNB + 8;
   const int64_t k = n;
@@ -1564,8 +1323,7 @@ __global__ void tsvd_add_kernel(cplx* __restrict__ base, long long chain_stride,
 void qr(const Arena& a, int64_t A, int64_t Q, int64_t R, int64_t work, int64_t m, int64_t n);
 
 bool qr_blocked(const Arena& a, int64_t A, int64_t Q, int64_t R, int64_t work, int64_t m, int64_t n) {
-  static const bool on = !(getenv("KBP_QR_BLOCKED") && atoi(getenv("KBP_QR_BLOCKED")) == 0);
-  if (!on || a.mask != nullptr || m < n || n < 128) return false;
+  if (a.mask != nullptr || m < n || n < 128) return false;
   const int64_t nblocks = (n + 63) / 64;
   const int64_t w = ((n + nblocks - 1) / nblocks + 7) / 8 * 8;         // block width: <= 64, multiple of 8, no tiny last block
   const int64_t Qt = work, V = Qt + n * m, Qj = V + m * w, C1 = Qj + m * w, C2 = C1 + n * w, Rjj = C2 + n * w, wk = Rjj + w * w;
@@ -1613,7 +1371,6 @@ bool qr_blocked(const Arena& a, int64_t A, int64_t Q, int64_t R, int64_t work, i
 }
 
 void init_tsvd_attributes() {
-  cudaFuncSetAttribute(cholqr_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 217 * 1024);   // + 8 KB static shared memory <= 227 KB
   cudaFuncSetAttribute(chol_reg_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
   cudaFuncSetAttribute(chol_reg_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
   cudaFuncSetAttribute(chol_reg_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 217 * 1024);

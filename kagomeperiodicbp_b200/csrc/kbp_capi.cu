@@ -34,8 +34,7 @@ struct kbp_ctx {
   kbp::SvdCtl* ctl = nullptr;            // device control block of the truncation in flight, followed by int state[nb]
   kbp::SvdCtl* ctl_host = nullptr;       // pinned mirror (host-driven mode, counters)
   cudaStream_t body_stream[2] = {nullptr, nullptr};   // capture streams of conditional-node bodies
-  // a program can be held as a LIST of graphs launched back to back (KBP_GRAPH_SEGMENT_LAUNCHES; off by default, see kbp_run)
-  struct GraphEntry { cudaGraphExec_t exec = nullptr; std::vector<cudaGraphExec_t> more; int seen = 0; int64_t launches = 0; int64_t dcount[8] = {0}; double flops = 0; bool bad = false; bool spec = false; };
+  struct GraphEntry { cudaGraphExec_t exec = nullptr; int seen = 0; int64_t launches = 0; int64_t dcount[8] = {0}; double flops = 0; bool bad = false; bool spec = false; };
   std::unordered_map<uint64_t, GraphEntry> graphs;      // CUDA graphs of whole programs, keyed by a hash of the op stream
   std::unordered_map<unsigned long long, int> tsvd_rounds;
   int64_t graph_replays = 0;
@@ -116,9 +115,7 @@ int kbp_create(int device, kbp_ctx** out) {
 
 static void drop_entry_graphs(kbp_ctx::GraphEntry& ge) {
   if (ge.exec) cudaGraphExecDestroy(ge.exec);
-  for (auto e : ge.more) cudaGraphExecDestroy(e);
   ge.exec = nullptr;
-  ge.more.clear();
 }
 
 static void drop_graphs(kbp_ctx* c) {
@@ -343,10 +340,7 @@ static inline double bits_to_double(int64_t b) {
   return d;
 }
 
-// runs the ops from word *pos (nullptr: 0) on; with max_launches > 0 it stops at the first op boundary after that many kernel
-// launches and leaves the position of the next op in *pos (== n_words: program finished)
-static int run_ops(kbp_ctx* c, const int64_t* w, int64_t n_words, bool capture, cudaGraph_t top_graph, uint64_t phash, int64_t* pos = nullptr,
-                   int64_t max_launches = 0);
+static int run_ops(kbp_ctx* c, const int64_t* w, int64_t n_words, bool capture, cudaGraph_t top_graph, uint64_t phash);
 
 static uint64_t program_hash(const int64_t* w, int64_t n_words) {
   uint64_t h = 1469598103934665603ull;
@@ -380,8 +374,6 @@ int kbp_run(kbp_ctx* c, const int64_t* w, int64_t n_words) {
   if (!c || !c->arena || !w) return fail(c, KBP_E_ARG, "kbp_run: arena not reserved");
   static const bool graphs_on = kbp::graphs_enabled();
   static const bool sync_every = getenv("KBP_SYNC_EVERY_OP") != nullptr;
-  static const bool env_first = getenv("KBP_GRAPH_FIRST") != nullptr && atoi(getenv("KBP_GRAPH_FIRST")) != 0;
-  const bool capture_first = env_first || c->graph_first;
   const uint64_t h = program_hash(w, n_words);
   c->last_run_spec = false;
   if (!graphs_on || c->profile || sync_every || n_words < c->graph_min_words) return run_ops(c, w, n_words, false, nullptr, h);
@@ -396,7 +388,6 @@ int kbp_run(kbp_ctx* c, const int64_t* w, int64_t n_words) {
   CU(c, cudaMemsetAsync(reinterpret_cast<char*>(c->ctl) + offsetof(kbp::SvdCtl, spec_fail), 0, sizeof(int), c->stream));
   if (ge.exec) {
     CU(c, cudaGraphLaunch(ge.exec, c->stream));
-    for (auto e : ge.more) CU(c, cudaGraphLaunch(e, c->stream));
     c->last_run_spec = ge.spec;
     c->spec_launches += ge.spec;
     c->launches += ge.launches;
@@ -405,7 +396,7 @@ int kbp_run(kbp_ctx* c, const int64_t* w, int64_t n_words) {
     ++c->graph_replays;
     return KBP_OK;
   }
-  if (ge.bad || (ge.seen++ == 0 && !capture_first)) return run_ops(c, w, n_words, false, nullptr, h);
+  if (ge.bad || (ge.seen++ == 0 && !c->graph_first)) return run_ops(c, w, n_words, false, nullptr, h);
   const int64_t l0 = c->launches;
   const double f0 = c->gemm_flops;
   int64_t c0[8];
@@ -419,49 +410,39 @@ int kbp_run(kbp_ctx* c, const int64_t* w, int64_t n_words) {
     fprintf(stderr, "[kbp] graph capture of a %lld-word program failed (%s): running it with host-driven loops\n", (long long)n_words, why);
     return run_ops(c, w, n_words, false, nullptr, h);
   };
-  // 0 = one graph per program (default).  Cutting a program into graphs of a few thousand launches was measured to be far WORSE:
-  // the launch call of the second graph on a stream blocks the host while the first is executing (N = 6 block: 226 ms per
-  // call instead of 20-30 ms; six sides 1574 ms instead of 685 ms per BP iteration).
-  static const int64_t seg_launches = getenv("KBP_GRAPH_SEGMENT_LAUNCHES") ? atoll(getenv("KBP_GRAPH_SEGMENT_LAUNCHES")) : 0;
-  std::vector<cudaGraphExec_t> execs;
-  int64_t pos = 0;
-  while (pos < n_words) {
-    if (cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) { for (auto e : execs) cudaGraphExecDestroy(e); return give_up("begin capture"); }
-    cudaStreamCaptureStatus st;
-    unsigned long long id;
-    cudaGraph_t top = nullptr;
-    const cudaGraphNode_t* deps = nullptr;
-    size_t nd = 0;
-    int rc = KBP_E_CUDA;
-    const int64_t pos0 = pos;
-    if (cudaStreamGetCaptureInfo_v2(c->stream, &st, &id, &top, &deps, &nd) == cudaSuccess && top) rc = run_ops(c, w, n_words, true, top, h, &pos, seg_launches);
-    cudaGraph_t graph = nullptr;
-    const cudaError_t e1 = cudaStreamEndCapture(c->stream, &graph);
-    if (rc != KBP_OK || e1 != cudaSuccess || !graph || pos <= pos0) {
-      for (int k = 0; k < 2; ++k) {                      // a body capture left open by a failure inside an op
-        cudaStreamCaptureStatus bs;
-        if (cudaStreamIsCapturing(c->body_stream[k], &bs) == cudaSuccess && bs != cudaStreamCaptureStatusNone) { cudaGraph_t g2 = nullptr; cudaStreamEndCapture(c->body_stream[k], &g2); }
-      }
-      if (graph) cudaGraphDestroy(graph);
-      for (auto e : execs) cudaGraphExecDestroy(e);
-      return give_up(rc != KBP_OK ? c->err.c_str() : cudaGetErrorString(e1));
+  // One graph per program.  Cutting a program into graphs of a few thousand launches was measured to be far WORSE: the launch
+  // call of the second graph on a stream blocks the host while the first is executing (N = 6 block: 226 ms per call instead
+  // of 20-30 ms; six sides 1574 ms instead of 685 ms per BP iteration).
+  if (n_words == 0) return give_up("empty program");
+  if (cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) return give_up("begin capture");
+  cudaStreamCaptureStatus st;
+  unsigned long long id;
+  cudaGraph_t top = nullptr;
+  const cudaGraphNode_t* deps = nullptr;
+  size_t nd = 0;
+  int rc = KBP_E_CUDA;
+  if (cudaStreamGetCaptureInfo_v2(c->stream, &st, &id, &top, &deps, &nd) == cudaSuccess && top) rc = run_ops(c, w, n_words, true, top, h);
+  cudaGraph_t graph = nullptr;
+  const cudaError_t e1 = cudaStreamEndCapture(c->stream, &graph);
+  if (rc != KBP_OK || e1 != cudaSuccess || !graph) {
+    for (int k = 0; k < 2; ++k) {                        // a body capture left open by a failure inside an op
+      cudaStreamCaptureStatus bs;
+      if (cudaStreamIsCapturing(c->body_stream[k], &bs) == cudaSuccess && bs != cudaStreamCaptureStatusNone) { cudaGraph_t g2 = nullptr; cudaStreamEndCapture(c->body_stream[k], &g2); }
     }
-    cudaGraphExec_t ex = nullptr;
-    const cudaError_t e2 = cudaGraphInstantiate(&ex, graph, 0);
-    cudaGraphDestroy(graph);
-    if (e2 != cudaSuccess) { for (auto e : execs) cudaGraphExecDestroy(e); return give_up(cudaGetErrorString(e2)); }
-    execs.push_back(ex);
+    if (graph) cudaGraphDestroy(graph);
+    return give_up(rc != KBP_OK ? c->err.c_str() : cudaGetErrorString(e1));
   }
-  if (execs.empty()) return give_up("empty program");
-  ge.exec = execs[0];
-  ge.more.assign(execs.begin() + 1, execs.end());
+  cudaGraphExec_t ex = nullptr;
+  const cudaError_t e2 = cudaGraphInstantiate(&ex, graph, 0);
+  cudaGraphDestroy(graph);
+  if (e2 != cudaSuccess) return give_up(cudaGetErrorString(e2));
+  ge.exec = ex;
   ge.launches = c->launches - l0;
   ge.flops = c->gemm_flops - f0;
   for (int k = 0; k < 8; ++k) ge.dcount[k] = c->counters[k] - c0[k];
   ge.spec = c->speculate;
   ++c->graph_captures;
   CU(c, cudaGraphLaunch(ge.exec, c->stream));
-  for (auto e : ge.more) CU(c, cudaGraphLaunch(e, c->stream));
   c->last_run_spec = ge.spec;
   c->spec_launches += ge.spec;
   ++c->graph_replays;
@@ -523,7 +504,7 @@ int kbp_spec_counters(const kbp_ctx* c, int64_t* out2) {
   return KBP_OK;
 }
 
-static int run_ops(kbp_ctx* c, const int64_t* w, int64_t n_words, bool capture, cudaGraph_t top_graph, uint64_t phash, int64_t* pos, int64_t max_launches) {
+static int run_ops(kbp_ctx* c, const int64_t* w, int64_t n_words, bool capture, cudaGraph_t top_graph, uint64_t phash) {
   if (!c || !c->arena || !w) return fail(c, KBP_E_ARG, "kbp_run: arena not reserved");
   CU(c, cudaSetDevice(c->device));
   kbp::Arena a;
@@ -537,12 +518,10 @@ static int run_ops(kbp_ctx* c, const int64_t* w, int64_t n_words, bool capture, 
   const int64_t E = c->chain_elems;
   auto in_arena = [&](int64_t off, int64_t n) { return off >= 0 && n >= 0 && off + n <= E; };
   auto slot_ok = [&](int64_t s) { return s >= -1 && s < c->n_slots; };
-  int64_t i = pos ? *pos : 0;
-  const int64_t launches_at_start = c->launches;
+  int64_t i = 0;
   const int status = KBP_OK;
   static const bool sync_every = getenv("KBP_SYNC_EVERY_OP") != nullptr;
   while (i < n_words) {
-    if (max_launches > 0 && c->launches - launches_at_start >= max_launches) break;
     const int64_t op = w[i];
     char where[64];
     snprintf(where, sizeof(where), " (op %lld at word %lld)", (long long)op, (long long)i);
@@ -682,7 +661,6 @@ static int run_ops(kbp_ctx* c, const int64_t* w, int64_t n_words, bool capture, 
   }
 #undef NEED
 #undef BAD
-  if (pos) *pos = i;
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail(c, KBP_E_CUDA, std::string("kernel launch: ") + cudaGetErrorString(e));
   return status;
