@@ -31,6 +31,8 @@ def _op(a, rows, cols, op):
 class NumpyEngine:
     """duck-types kagomeperiodicbp_b200.engine.Engine"""
 
+    svd_input_norms = None               # a list: every OP_SVD appends the Frobenius norm of its input (input norm survey)
+
     def __init__(self):
         self.nb = 0
         self.n_slots = 0
@@ -137,6 +139,8 @@ class NumpyEngine:
                 A, US, Vh, wk, m, n, keep, nrb, s0, s1, warm = w[i + 1:i + 12]
                 u, s, vh = np.linalg.svd(ar[A:A + m * n].reshape(m, n), full_matrices=False)
                 fro = np.linalg.norm(s)
+                if NumpyEngine.svd_input_norms is not None:
+                    NumpyEngine.svd_input_norms.append(float(fro))
                 if s1 >= 0 and fro > 0:
                     sl[s1] += math.sqrt(np.sum(s[keep:] ** 2) / np.sum(s ** 2))
                 if nrb and fro > 0:

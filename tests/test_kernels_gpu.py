@@ -71,7 +71,9 @@ def test_tensordot_conj(eng):
 @pytest.mark.parametrize("m,n", [(5, 3), (3, 5), (16, 16), (162, 18), (18, 162), (512, 32), (64, 64), (1, 4), (4, 1), (256, 32), (768, 48),
                                  (243, 27), (256, 16), (130, 7), (1024, 40), (1100, 16), (96, 200),
                                  (1024, 64), (2592, 72), (2000, 40), (1300, 130),        # TSQR over row blocks / one-CTA kernel
-                                 (672, 672), (300, 200), (700, 129)])                     # large, not skinny: block Gram-Schmidt over tall-skinny blocks
+                                 (672, 672), (392, 392), (816, 264),                      # large, not skinny: block Gram-Schmidt over tall-skinny blocks
+                                 (300, 200), (700, 129), (384, 384),                      # too little workspace for the blocked path: Householder
+                                 (208, 32), (207, 32), (592, 96), (584, 96), (300, 8), (300, 7)])   # Cholesky-QR2 at its workspace and width edges
 def test_qr(eng, m, n):
     batch = [[rnd(m, n)] for _ in range(3)]
     # make one of them rank deficient
@@ -221,8 +223,9 @@ def test_svd_subspace_wide_block_two_column_blocks(eng, m, n, keep):
 
 
 def test_svd_subspace_widest_block(eng):
-    """keep = 42 (chi = 2 D^2 + 10 at D = 4: the ToCore / ToEdge chains) runs the subspace path with the widest block the
-    b x b kernels take (112): their shared-memory footprints must fit."""
+    """keep = 42 (chi = 2 D^2 + 10 at D = 4: the ToCore / ToEdge chains) runs the subspace path with a block of 88 columns
+    (the register Cholesky of up to 96 columns).  The widest one-block panel (112, chol_blocked_kernel) is reached by keep 49-56
+    in test_kernel_routes_gpu.py."""
     m, n, keep = 672, 672, 42
     a = rnd(m, n)
     u, s, vh = np.linalg.svd(a, full_matrices=False)
