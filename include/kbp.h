@@ -88,22 +88,8 @@ int kbp_graph_ready(kbp_ctx* ctx, const int64_t* words, int64_t n_words);
 /* programs shorter than min_words are never captured (default 256); capture_first != 0: capture at first sight (default: second) */
 int kbp_graph_policy(kbp_ctx* ctx, int64_t min_words, int capture_first);
 int kbp_sync(kbp_ctx* ctx);
-/* SPECULATIVE program graphs (opt-in: KBP_SPECULATE=1 or kbp_set_speculation(ctx, 1)).  A captured program gives each truncated
- * SVD whose host-driven run was settled by the subspace iteration a FIXED schedule (the iterations it needed + one) and no
- * WHILE / IF node.  Every truncation still runs its acceptance test; a miss raises a sticky device flag.  Protocol: after the
- * program (kbp_run) and before using anything it wrote, call kbp_spec_failed (waits for the stream); if it returns 1, call
- * kbp_run_relearn with the same words -- inputs are never overwritten by a program, so they are still in place -- which runs
- * the program host-driven with every data-dependent loop and exact fallback, records the new schedule and drops the stale
- * graph.  kbp_spec_counters: out2[0] speculative graph launches, [1] failed ones.  Measured on the B200 (six side programs of
- * the D = 4, N = 6 block side by side): 648 ms per BP iteration against 672 ms with the conditional nodes -- and a schedule
- * learned from staged rounds misses its test now and then even on unchanged inputs, which costs a host-driven rerun; hence
- * off by default.  With speculation off kbp_spec_failed always returns 0. */
-int kbp_spec_failed(kbp_ctx* ctx);
-int kbp_run_relearn(kbp_ctx* ctx, const int64_t* words, int64_t n_words);
-int kbp_set_speculation(kbp_ctx* ctx, int on);
 /* developer probe (KBP_KTIME=1 in the environment): print and reset the in-kernel wall time of the Cholesky CTAs */
 int kbp_ktime_report(kbp_ctx* ctx, const char* tag);
-int kbp_spec_counters(const kbp_ctx* ctx, int64_t* out2);
 
 /* device addresses of the arena ([nb][chain_elems] complex128), of the slot table ([nb][n_slots] doubles) and the CUDA stream
  * handle of the context, for zero-copy exchange of block messages between the arenas of different GPUs (NCCL all-gather in

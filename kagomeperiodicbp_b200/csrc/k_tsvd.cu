@@ -945,7 +945,7 @@ constexpr double TSVD_PIVOT_TRUST = 1e-3;
 __global__ void tsvd_decide_kernel(SvdCtl* __restrict__ ctl, int* __restrict__ state, double* __restrict__ stat, const double* __restrict__ resid,
                                    const double* __restrict__ ratio, const double* __restrict__ discf, int nb, int first, int max_rounds,
                                    int iters_first, int iters_more, cudaGraphConditionalHandle h_loop, cudaGraphConditionalHandle h_exact,
-                                   int use_handles, int spec, const cplx* __restrict__ base, long long chain_stride, long long R1_, int b, int keep) {
+                                   int use_handles, const cplx* __restrict__ base, long long chain_stride, long long R1_, int b, int keep) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   const int round = first ? 1 : ctl->round + 1;
   int any_run = 0, any_exact = 0;
@@ -988,7 +988,6 @@ __global__ void tsvd_decide_kernel(SvdCtl* __restrict__ ctl, int* __restrict__ s
     cudaGraphSetConditional(h_loop, any_run ? 1u : 0u);
     cudaGraphSetConditional(h_exact, any_exact ? 1u : 0u);
   }
-  if (spec && (any_run || any_exact)) ctl->spec_fail = 1;        // speculative graph: nothing follows up on this op; the run is void
 }
 
 int svd_exact(const Arena& a, int64_t A, int64_t US, int64_t Vh, int64_t work, int64_t m, int64_t n, int64_t keep, int nr_bulk,
@@ -1100,7 +1099,7 @@ static void tsvd_more_round(const Arena& a, const TsvdBufs& w, int64_t A, int64_
   // TSVD_IT_MORE odd: cur == Qb again
   rayleigh_ritz_and_check(a, w, A, US, Vh, m, n, keep, b, cur, f0, f1, true);
   tsvd_decide_kernel<<<1, 32, 0, a.stream>>>(a.ctl, a.chain_state, stat, a.svd_off + a.nb, a.svd_off + 2 * a.nb, a.svd_off + 3 * a.nb, a.nb, 0,
-                                             max_rounds, iters_first, TSVD_IT_MORE, h_loop, h_exact, a.capture ? 1 : 0, 0, a.base, a.chain_stride, w.R1, b, (int)keep);
+                                             max_rounds, iters_first, TSVD_IT_MORE, h_loop, h_exact, a.capture ? 1 : 0, a.base, a.chain_stride, w.R1, b, (int)keep);
   ++*a.launches;
 }
 
@@ -1109,12 +1108,6 @@ constexpr int TSVD_IT_COLD = 7;
 // cold start: after TSVD_SAFE_ITERS SAFE iterations the block is already ordered well enough (contamination of column j by a
 // larger direction i has decayed as (s_j/s_i)^(2k), one fast step amplifies it by (s_i/s_j)^2) for the FAST form
 constexpr int TSVD_SAFE_ITERS = 2;
-// SPECULATIVE capture (Arena::speculate): an op whose host-driven run was settled by the subspace iteration within four
-// rounds gets that schedule plus TSVD_SPEC_SLACK iterations and NO conditional node -- a conditional node makes the GPU drain
-// every kernel in flight, also those of the other program graphs running beside this one (six side programs: each of the
-// ~550 nodes per chain waited for some other chain's 300 us Jacobi kernel).  The acceptance test still runs; a miss
-// raises SvdCtl::spec_fail and the host reruns the program host-driven, which also re-learns the schedule.
-constexpr int TSVD_SPEC_SLACK = 1;
 
 // Two kinds of iteration.  SAFE (cold start, Q arbitrary): W = A Q, Y = orth(W), Z = A^H Y, Q = orth(Z).  FAST (Q holds
 // approximate Ritz vectors in decreasing order -- after TSVD_SAFE_ITERS SAFE iterations of a cold start, or after a Rayleigh-Ritz
@@ -1131,14 +1124,9 @@ int svd_truncate_subspace(const Arena& a0, int64_t A, int64_t US, int64_t Vh, in
   // An op that needed r > 1 rounds when its program ran host-driven (previous BP iteration: nearly the same spectrum) gets
   // the iterations of those rounds up front in the captured graph: one Rayleigh-Ritz step + check instead of r.
   int it_cold = TSVD_IT_COLD;
-  bool spec = false;
   if (a0.capture && a0.tsvd_rounds) {
     auto f = a0.tsvd_rounds->find(a0.op_key);
     if (f != a0.tsvd_rounds->end() && f->second > 1) it_cold = TSVD_IT_COLD + ((f->second < 4 ? f->second : 4) - 1) * TSVD_IT_MORE;
-    if (a0.speculate && f != a0.tsvd_rounds->end() && f->second >= 1 && f->second <= 4) {
-      spec = true;
-      it_cold += TSVD_SPEC_SLACK;
-    }
   }
   // a block narrower than 2.5 keep converges more slowly: more iterations are still far cheaper than the exact path
   const int it_max = 2 * b >= 5 * keep ? 24 : 72;
@@ -1162,7 +1150,7 @@ int svd_truncate_subspace(const Arena& a0, int64_t A, int64_t US, int64_t Vh, in
   w.Pb = o;               // m x n: P = US Vh
   double* stat = a.svd_off;          // [nb] min pivot ratio, then [nb] each: residual, ratio, discarded fraction, [2 nb] norms, partial sums
   double* norms = a.svd_off + 4 * a.nb;
-  const cudaGraphConditionalHandle h_loop = spec ? 0 : new_cond_handle(a), h_exact = spec ? 0 : new_cond_handle(a);
+  const cudaGraphConditionalHandle h_loop = new_cond_handle(a), h_exact = new_cond_handle(a);
 
   // ---- round 1: pseudo-random block, it_cold iterations
   int64_t Qb = w.panel[0], f0 = w.panel[1], f1 = w.panel[2], f2 = w.panel[3];
@@ -1210,14 +1198,13 @@ int svd_truncate_subspace(const Arena& a0, int64_t A, int64_t US, int64_t Vh, in
   }
   rayleigh_ritz_and_check(a, w, A, US, Vh, m, n, keep, b, Qb, f0, f1, cold_fast);
   tsvd_decide_kernel<<<1, 32, 0, a.stream>>>(a.ctl, a.chain_state, stat, a.svd_off + a.nb, a.svd_off + 2 * a.nb, a.svd_off + 3 * a.nb, a.nb, 1,
-                                             max_rounds, it_cold, TSVD_IT_MORE, h_loop, h_exact, (a.capture && !spec) ? 1 : 0, spec ? 1 : 0, a.base, a.chain_stride, w.R1,
+                                             max_rounds, it_cold, TSVD_IT_MORE, h_loop, h_exact, a.capture ? 1 : 0, a.base, a.chain_stride, w.R1,
                                              b, (int)keep);
   ++*a.launches;
 
   // ---- further rounds while some chain is RUNNING; only those chains take part
   int rounds = 1;
-  if (spec) {
-  } else if (a.capture) {
+  if (a.capture) {
     Arena body;
     if (!begin_cond_body(a, h_loop, true, &body)) return -1;
     body.mask = a.chain_state; body.mask_want = CHAIN_RUNNING;
@@ -1242,8 +1229,7 @@ int svd_truncate_subspace(const Arena& a0, int64_t A, int64_t US, int64_t Vh, in
   ++*a.launches;
   // ---- chains the iteration could not settle: exact block-Jacobi SVD of the same matrix
   bool used_exact = false;
-  if (spec) {
-  } else if (a.capture) {
+  if (a.capture) {
     Arena body;
     if (!begin_cond_body(a, h_exact, false, &body)) return -1;
     body.mask = a.chain_state; body.mask_want = CHAIN_EXACT;

@@ -34,14 +34,11 @@ struct kbp_ctx {
   kbp::SvdCtl* ctl = nullptr;            // device control block of the truncation in flight, followed by int state[nb]
   kbp::SvdCtl* ctl_host = nullptr;       // pinned mirror (host-driven mode, counters)
   cudaStream_t body_stream[2] = {nullptr, nullptr};   // capture streams of conditional-node bodies
-  struct GraphEntry { cudaGraphExec_t exec = nullptr; int seen = 0; int64_t launches = 0; int64_t dcount[8] = {0}; double flops = 0; bool bad = false; bool spec = false; };
+  struct GraphEntry { cudaGraphExec_t exec = nullptr; int seen = 0; int64_t launches = 0; int64_t dcount[8] = {0}; double flops = 0; bool bad = false; };
   std::unordered_map<uint64_t, GraphEntry> graphs;      // CUDA graphs of whole programs, keyed by a hash of the op stream
   std::unordered_map<unsigned long long, int> tsvd_rounds;
   int64_t graph_replays = 0;
   int64_t graph_captures = 0;
-  bool speculate = false;                // captured programs are speculative (no conditional nodes on learned truncations): opt-in, KBP_SPECULATE=1
-  bool last_run_spec = false;            // the program in flight on the stream is such a graph
-  int64_t spec_launches = 0, spec_failures = 0;
   int64_t graph_min_words = 256;         // shorter programs (one-off algebra of the ITE step) run as plain launches
   bool graph_first = false;              // capture a program the first time it is seen (default: the second)
   bool profile = false;
@@ -105,7 +102,6 @@ int kbp_create(int device, kbp_ctx** out) {
   }
   // blocking host waits on request (KBP_BLOCKING_SYNC=1): useful when many ranks share few host cores; measured on a
   // 4 x B200 / 32-core box the default spin wait is ~6 % faster, so it stays the default
-  if (const char* sp = getenv("KBP_SPECULATE")) c->speculate = atoi(sp) != 0;
   const char* bs = getenv("KBP_BLOCKING_SYNC");
   const bool blocking = bs && atoi(bs) != 0;
   if (blocking && cudaEventCreateWithFlags(&c->block_event, cudaEventBlockingSync | cudaEventDisableTiming) != cudaSuccess) c->block_event = nullptr;
@@ -113,13 +109,9 @@ int kbp_create(int device, kbp_ctx** out) {
   return KBP_OK;
 }
 
-static void drop_entry_graphs(kbp_ctx::GraphEntry& ge) {
-  if (ge.exec) cudaGraphExecDestroy(ge.exec);
-  ge.exec = nullptr;
-}
-
 static void drop_graphs(kbp_ctx* c) {
-  for (auto& kv : c->graphs) drop_entry_graphs(kv.second);
+  for (auto& kv : c->graphs)
+    if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
   c->graphs.clear();
 }
 
@@ -366,6 +358,16 @@ int kbp_graph_ready(kbp_ctx* c, const int64_t* w, int64_t n_words) {
   return !it->second.bad && (it->second.exec != nullptr || it->second.seen >= 1 || c->graph_first);
 }
 
+// launch the graph of a captured program and count its launches, GEMM flops and host-decided SVD routes
+static int launch_graph(kbp_ctx* c, const kbp_ctx::GraphEntry& ge) {
+  CU(c, cudaGraphLaunch(ge.exec, c->stream));
+  c->launches += ge.launches;
+  c->gemm_flops += ge.flops;
+  for (int k = 0; k < 2; ++k) c->counters[k] += ge.dcount[k];
+  ++c->graph_replays;
+  return KBP_OK;
+}
+
 // Every program is a CUDA graph from its second run on: the op stream is a constant launch sequence except for the
 // truncated SVDs, whose data-dependent loops are captured as conditional WHILE / IF nodes driven by one-thread decision
 // kernels (k_tsvd.cu, k_svd.cu).  The first run is host-driven (plain launches, control block read back per decision): it
@@ -375,7 +377,6 @@ int kbp_run(kbp_ctx* c, const int64_t* w, int64_t n_words) {
   static const bool graphs_on = kbp::graphs_enabled();
   static const bool sync_every = getenv("KBP_SYNC_EVERY_OP") != nullptr;
   const uint64_t h = program_hash(w, n_words);
-  c->last_run_spec = false;
   if (!graphs_on || c->profile || sync_every || n_words < c->graph_min_words) return run_ops(c, w, n_words, false, nullptr, h);
   auto it = c->graphs.find(h);
   if (it == c->graphs.end()) {
@@ -384,29 +385,21 @@ int kbp_run(kbp_ctx* c, const int64_t* w, int64_t n_words) {
   }
   kbp_ctx::GraphEntry& ge = it->second;
   CU(c, cudaSetDevice(c->device));
-  c->last_run_spec = false;
-  CU(c, cudaMemsetAsync(reinterpret_cast<char*>(c->ctl) + offsetof(kbp::SvdCtl, spec_fail), 0, sizeof(int), c->stream));
-  if (ge.exec) {
-    CU(c, cudaGraphLaunch(ge.exec, c->stream));
-    c->last_run_spec = ge.spec;
-    c->spec_launches += ge.spec;
-    c->launches += ge.launches;
-    c->gemm_flops += ge.flops;
-    for (int k = 0; k < 2; ++k) c->counters[k] += ge.dcount[k];
-    ++c->graph_replays;
-    return KBP_OK;
-  }
+  if (ge.exec) return launch_graph(c, ge);
   if (ge.bad || (ge.seen++ == 0 && !c->graph_first)) return run_ops(c, w, n_words, false, nullptr, h);
   const int64_t l0 = c->launches;
   const double f0 = c->gemm_flops;
   int64_t c0[8];
   for (int k = 0; k < 8; ++k) c0[k] = c->counters[k];
-  auto give_up = [&](const char* why) {
-    ge.bad = true;
-    cudaGetLastError();
+  auto restore_counters = [&] {
     c->launches = l0;
     c->gemm_flops = f0;
     for (int k = 0; k < 8; ++k) c->counters[k] = c0[k];
+  };
+  auto give_up = [&](const char* why) {
+    ge.bad = true;
+    cudaGetLastError();
+    restore_counters();
     fprintf(stderr, "[kbp] graph capture of a %lld-word program failed (%s): running it with host-driven loops\n", (long long)n_words, why);
     return run_ops(c, w, n_words, false, nullptr, h);
   };
@@ -440,45 +433,9 @@ int kbp_run(kbp_ctx* c, const int64_t* w, int64_t n_words) {
   ge.launches = c->launches - l0;
   ge.flops = c->gemm_flops - f0;
   for (int k = 0; k < 8; ++k) ge.dcount[k] = c->counters[k] - c0[k];
-  ge.spec = c->speculate;
+  restore_counters();                                    // capturing ran nothing: launch_graph counts the first run
   ++c->graph_captures;
-  CU(c, cudaGraphLaunch(ge.exec, c->stream));
-  c->last_run_spec = ge.spec;
-  c->spec_launches += ge.spec;
-  ++c->graph_replays;
-  return KBP_OK;
-}
-
-// 1: the program last started by kbp_run was a speculative graph and one of its truncations missed its acceptance test, so
-// nothing it wrote may be used: call kbp_run_relearn with the same words (inputs are still in place), then read the results.
-// Waits for the stream.  0: results valid.
-int kbp_spec_failed(kbp_ctx* c) {
-  if (!c || !c->ctl || !c->ctl_host) return 0;
-  if (!c->last_run_spec) return 0;
-  cudaSetDevice(c->device);
-  if (cudaMemcpyAsync(c->ctl_host, c->ctl, sizeof(kbp::SvdCtl), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) return 0;
-  if (ctx_wait(c) != cudaSuccess) return 0;
-  const int f = c->ctl_host->spec_fail != 0;
-  if (f) ++c->spec_failures;
-  c->last_run_spec = false;
-  return f;
-}
-
-// run the program host-driven (every data-dependent loop decided from the control block, exact fallbacks included), which
-// records what each truncation needed, and forget its graph: the next kbp_run captures it again with the new schedule
-int kbp_run_relearn(kbp_ctx* c, const int64_t* w, int64_t n_words) {
-  if (!c || !c->arena || !w) return fail(c, KBP_E_ARG, "kbp_run_relearn: arena not reserved");
-  CU(c, cudaSetDevice(c->device));
-  const uint64_t h = program_hash(w, n_words);
-  auto it = c->graphs.find(h);
-  if (it != c->graphs.end()) {
-    CU(c, cudaStreamSynchronize(c->stream));
-    drop_entry_graphs(it->second);
-    it->second.seen = 1;                               // the run below is its host-driven sighting
-  }
-  c->last_run_spec = false;
-  CU(c, cudaMemsetAsync(reinterpret_cast<char*>(c->ctl) + offsetof(kbp::SvdCtl, spec_fail), 0, sizeof(int), c->stream));
-  return run_ops(c, w, n_words, false, nullptr, h);
+  return launch_graph(c, ge);
 }
 
 /* developer probe (KBP_KTIME=1): prints and resets the in-kernel timing of the Cholesky CTAs (k_tsvd.cu) */
@@ -487,20 +444,6 @@ int kbp_ktime_report(kbp_ctx* c, const char* tag) {
   cudaSetDevice(c->device);
   cudaDeviceSynchronize();
   kbp::ktime_report(tag ? tag : "");
-  return KBP_OK;
-}
-
-int kbp_set_speculation(kbp_ctx* c, int on) {
-  if (!c) return KBP_E_ARG;
-  c->speculate = on != 0;
-  return KBP_OK;
-}
-
-// out2: speculative graph launches, those that failed their acceptance tests
-int kbp_spec_counters(const kbp_ctx* c, int64_t* out2) {
-  if (!c || !out2) return KBP_E_ARG;
-  out2[0] = c->spec_launches;
-  out2[1] = c->spec_failures;
   return KBP_OK;
 }
 
@@ -514,7 +457,7 @@ static int run_ops(kbp_ctx* c, const int64_t* w, int64_t n_words, bool capture, 
   a.ctl = c->ctl; a.ctl_host = c->ctl_host; a.chain_state = reinterpret_cast<int*>(c->ctl + 1);
   a.mask = nullptr; a.mask_want = 0;
   a.tsvd_rounds = &c->tsvd_rounds; a.op_key = 0;
-  a.capture = capture; a.speculate = capture && c->speculate; a.top_graph = top_graph; a.body_stream[0] = c->body_stream[0]; a.body_stream[1] = c->body_stream[1]; a.depth = 0;
+  a.capture = capture; a.top_graph = top_graph; a.body_stream[0] = c->body_stream[0]; a.body_stream[1] = c->body_stream[1]; a.depth = 0;
   const int64_t E = c->chain_elems;
   auto in_arena = [&](int64_t off, int64_t n) { return off >= 0 && n >= 0 && off + n <= E; };
   auto slot_ok = [&](int64_t s) { return s >= -1 && s < c->n_slots; };

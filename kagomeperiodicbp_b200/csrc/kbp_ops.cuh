@@ -22,9 +22,7 @@ struct SvdCtl {
   int any_exact;           // some chain needs the exact path
   int sweeps;              // block-Jacobi sweeps done
   int any_sweep;           // some chain has not converged yet
-  int spec_fail;           // sticky: a truncation of a SPECULATIVE program graph (fixed schedule, no conditional nodes) missed its
-                           // acceptance test -- the results of the run are not to be used (kbp_spec_failed / kbp_run_relearn)
-  int pad[2];
+  int pad[3];
   long long counters[8];   // [2] truncations accepted from subspace iteration, [3] handed to the exact path, [4] exact-path runs,
                            // [5] subspace iterations, [6] block-Jacobi sweeps, [7] truncations that did not converge
 };
@@ -64,7 +62,6 @@ struct Arena {
   std::unordered_map<unsigned long long, int>* tsvd_rounds;
   unsigned long long op_key;
   bool capture;
-  bool speculate;         // capture only: truncations with a learned schedule get no WHILE / IF node (see SvdCtl::spec_fail)
   cudaGraph_t top_graph;
   cudaStream_t body_stream[2];
   int depth;

@@ -185,7 +185,6 @@ class ResidentBackend:
         self.arena_elems = arena_elems
         self.p = Program(8)
         self.eng.reserve(arena_elems, 1, 8)
-        self.eng.set_speculation(False)   # its programs are launched without the verify step of the speculative-graph protocol
         self.eng._loaded = None
         self.calls = 0
 

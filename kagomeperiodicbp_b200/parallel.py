@@ -119,8 +119,6 @@ class ShardedSides:
         torch = self.torch
         for s in self.mine:                                            # graph launches on the sides' own streams
             self.comps[s].run_resident(self.engs[s], (bp.E_SVD_NOCONV,))
-        for s in self.mine:                                            # speculative-graph protocol (include/kbp.h): before anything is gathered
-            self.comps[s].verify_resident(self.engs[s], (bp.E_SVD_NOCONV,))
         if self.on_cuda:
             main = self.stream
             for s in self.mine:

@@ -69,9 +69,6 @@ class Compiled:
 
     def collect(self, eng: Engine, nb: int, rc: int = 0):
         """second half of ``run``: ONE device->host copy of the packed outputs + the slot table (waits for the program)."""
-        if eng.spec_failed():                     # speculative graph missed an SVD acceptance test: host-driven rerun on the same inputs
-            eng.slots_zero()
-            rc = eng.run_relearn(self.words, soft_errors=(E_SVD_NOCONV,))
         raw = eng.download(self.out_block.off, self.out_elems)
         slots = eng.slots()
         if rc == 0 and slots.shape[1] and np.any(slots[:, -1] > 0):     # engine-reserved status slot (include/kbp.h)
@@ -96,14 +93,8 @@ class Compiled:
         return eng.run(self.words, soft_errors=soft_errors)
 
     def verify_resident(self, eng: Engine, soft_errors=()) -> bool:
-        """after ``run_resident``: wait for the program and, if it ran as a speculative graph that missed an SVD acceptance
-        test, rerun it host-driven (inputs are still resident).  Returns True when a rerun was needed."""
-        if not eng.spec_failed():
-            return False
-        eng.slots_zero()
-        eng.run_relearn(self.words, soft_errors=soft_errors)
-        eng.sync()
-        return True
+        """returns False (no rerun needed) and touches nothing: bench.py calls it after every ``run_resident``."""
+        return False
 
 
 _tls = threading.local()

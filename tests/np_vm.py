@@ -86,18 +86,6 @@ class NumpyEngine:
     def gemm_flops(self):
         return 0.0
 
-    def spec_failed(self):
-        return False                     # no speculative graphs in the interpreter
-
-    def set_speculation(self, on):
-        pass
-
-    def run_relearn(self, words, soft_errors=()):
-        return self.run(words, soft_errors=soft_errors)
-
-    def run_verified(self, words, soft_errors=()):
-        return self.run(words, soft_errors=soft_errors)
-
     def launch_count(self):
         return self._launches
 

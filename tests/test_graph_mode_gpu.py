@@ -165,27 +165,3 @@ def test_whole_side_program_as_graph():
         host.close()
         graph.close()
 
-
-def test_speculative_graph_protocol():
-    """opt-in speculative graphs (include/kbp.h: kbp_set_speculation / kbp_spec_failed / kbp_run_relearn): truncations with a
-    learned schedule get no conditional node; whatever the acceptance tests say on the device, what ``Compiled.run`` returns after
-    the verify step is the valid result -- on the inputs the schedule was learned on and on different ones (a harder spectrum
-    than the learned schedule covers must be caught by the flag and redone host-driven)."""
-    from kagomeperiodicbp_b200.engine import Engine
-    m, n, keep = 512, 512, 32
-    comp = compile_svd(m, n, keep)
-    easy = with_spectrum(m, n, np.sort(np.exp(-0.1 * np.arange(n)) * (1 + 0.3 * rng.random(n)))[::-1])
-    hard = with_spectrum(m, n, np.exp(-0.02 * np.arange(n)))          # needs several more rounds than `easy`
-    eng = Engine(0)
-    try:
-        eng.set_speculation(True)
-        eng.graph_policy(0, False)                                   # capture at the second sight of a program
-        for a in (easy, easy, easy, hard, hard, easy):
-            o, sl, rc = comp.run(eng, [{"i0": a}])
-            assert rc == 0
-            check(a, o[0]["o0"], o[0]["o1"], sl[0], keep)
-        sc = eng.spec_counters()
-        assert sc["spec_launches"] >= 1, sc
-        assert sc["spec_failures"] >= 1, sc                          # the first `hard` run on the `easy` schedule
-    finally:
-        eng.close()
