@@ -95,15 +95,16 @@ CORE_DIRECTIONS = {"U": ("U", "D", 0), "DL": ("DL", "UR", 4), "DR": ("DR", "UL",
 def core_env_tensors(B, N: int, mps_bottom_up, mps_top_down, direction: str = "U"):
     """zip the two ToCore boundary MPSs (bottom-up ``direction`` / its opposite) outside the core and return the 12 ring
     tensors m0..m11 (kagome_to_core.py:192-257; the ring is rotated by 0 / 4 / 8 places for U / DL / DR, :245-255).
-    Inputs: lists of site arrays [Dl, D^2, Dr]."""
+    Inputs: lists of site tensors [Dl, D^2, Dr] of the backend ``B`` (host arrays, or traced tensors of a compiled program).
+    The open end bonds are dropped with ``B.reshape``, so no site is read on the host."""
     s = 2 * N - 3
-    bu, td = [np.asarray(a) for a in mps_bottom_up], [np.asarray(a) for a in mps_top_down]
+    bu, td = list(mps_bottom_up), list(mps_top_down)
     assert len(bu) == 5 + 2 * s and len(td) == 7 + 2 * s, (len(bu), len(td))
     Lt = None
     for j in range(s):
         a, b = B.transpose(td[-j - 1], (2, 1, 0)), bu[j]
         if Lt is None:
-            Lt = B.tensordot(a[0], b[0], ([0], [0]))
+            Lt = B.tensordot(B.reshape(a, a.shape[1:]), B.reshape(b, b.shape[1:]), ([0], [0]))
         else:
             Lt = B.tensordot(B.tensordot(Lt, a, ([0], [0])), b, ([0, 1], [0, 1]))
     bu[s] = B.tensordot(Lt, bu[s], ([1], [0]))
@@ -111,7 +112,7 @@ def core_env_tensors(B, N: int, mps_bottom_up, mps_top_down, direction: str = "U
     for j in range(s):
         a, b = B.transpose(td[j], (2, 1, 0)), bu[-1 - j]
         if Rt is None:
-            Rt = B.tensordot(a[:, :, 0], b[:, :, 0], ([1], [1]))
+            Rt = B.tensordot(B.reshape(a, a.shape[:2]), B.reshape(b, b.shape[:2]), ([1], [1]))
         else:
             Rt = B.tensordot(B.tensordot(a, Rt, ([2], [0])), b, ([1, 2], [1, 2]))
     td[s] = B.tensordot(Rt, td[s], ([0], [0]))
@@ -129,7 +130,7 @@ def core_network(B, N: int, cell, env12):
     for k in range(9):
         # repeated unit cell: by flavor; non-repeated block (one tensor per lattice site): the core site's own tensor
         t = cell[flavor[tb[k]["name"]]] if len(cell) == 3 else cell[core_idx[k]]
-        kets[k] = (np.asarray(t), list(tb[k]["edges"]))
+        kets[k] = (t, list(tb[k]["edges"]))
     envs = {}
     for i in range(12):
         envs[i] = Node(env12[i], list(tb[9 + i]["edges"]))
@@ -241,8 +242,8 @@ def edge_environment(B, N: int, cell, env12, mode: str, edge: str, chi: int, bub
                 T_list.append(arrange(B, core.composite(core.resolve(n["name"], set())), n["edges"]).t)
         sites = bubblecon_fn(T_list, bc["edges"], bc["angles"], bc["bubble_angle"], bc["order"], chi, bc["kets"])
         assert len(sites) == 4
-        e01 = B.tensordot(sites[0][0], sites[1], ([1], [0]))            # [open0, open1, bond]
-        e32 = B.tensordot(sites[2], sites[3][:, :, 0], ([2], [0]))      # [bond, open2, open3]
+        e01 = B.tensordot(B.reshape(sites[0], sites[0].shape[1:]), sites[1], ([1], [0]))     # [open0, open1, bond]
+        e32 = B.tensordot(sites[2], B.reshape(sites[3], sites[3].shape[:2]), ([2], [0]))     # [bond, open2, open3]
         for pos, n in enumerate(ring_tbl):
             if n["name"] == "e-0+e-1":
                 ring[pos] = Node(e01, n["edges"])
@@ -279,8 +280,8 @@ def edge_environment(B, N: int, cell, env12, mode: str, edge: str, chi: int, bub
 
     # canonical leg order of the two sites, ring tensors with the D^2 leg opened to (ket, bra)
     pi, pj = et["perms"][et["nodes"][0]["name"]], et["perms"][et["nodes"][1]["name"]]
-    Ti = np.transpose(core.kets[ki][0], [0] + [1 + p for p in pi])
-    Tj = np.transpose(core.kets[kj][0], [0] + [1 + p for p in pj])
+    Ti = B.transpose(core.kets[ki][0], [0] + [1 + p for p in pi])
+    Tj = B.transpose(core.kets[kj][0], [0] + [1 + p for p in pj])
     D = Ti.shape[1]
     env = []
     for n in ring:
@@ -294,7 +295,12 @@ def edge_environment(B, N: int, cell, env12, mode: str, edge: str, chi: int, bub
     assert [n.legs[1] for n in ring] == ti_legs[1:] + tj_legs[1:], ([n.legs for n in ring], ti_legs, tj_legs)
     for a, b in zip(ring, ring[1:] + ring[:1]):
         assert a.legs[2] == b.legs[0] and a.t.shape[2] == b.t.shape[0], (a.legs, b.legs)
-    return np.ascontiguousarray(Ti), np.ascontiguousarray(Tj), env, dict(i=ki, j=kj, perm_i=pi, perm_j=pj, flavors=(core.flavor[ki], core.flavor[kj]))
+    return _contiguous(Ti), _contiguous(Tj), env, dict(i=ki, j=kj, perm_i=pi, perm_j=pj, flavors=(core.flavor[ki], core.flavor[kj]))
+
+
+def _contiguous(t):
+    """host arrays are returned C-contiguous; a traced tensor of a compiled program already is."""
+    return np.ascontiguousarray(t) if isinstance(t, np.ndarray) else t
 
 
 def write_back(cell, info, Ti_new, Tj_new):

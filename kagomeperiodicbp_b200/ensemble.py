@@ -75,8 +75,10 @@ def belief_propagation_batch(N: int, cells: list, config: BPConfig, messages_lis
 def run_ensemble(seeds, D: int, N: int, chi_factor: float = 1.0, rank: int = 0, world: int = 1, device: int = 0, batch: int = 8,
                  ite_steps: int = 0, delta_t: float = 1e-2, save_folder: str | None = None, method: int = 3, init: str = "random"):
     """one row per seed: random unit cell (method 3 of scripts/condor/send_ite.py:66-70) -> batched block BP -> `ite_steps` ITE
-    edge updates per cell -> energy per site.  ``init="su"``: the rank's random cells first go through one batched simple
-    update (simple_update.simple_update, default schedule) and BP starts from the SU cells.  Returns this rank's rows."""
+    edge updates per cell -> energy per site, measured for all the rank's cells by ``ite_flow.measure_energies_batch``
+    (``batch`` cells per launch; ``exec_time`` charges every cell an equal share of the batched BP and of the batched
+    measurement).  ``init="su"``: the rank's random cells first go through one batched simple update
+    (simple_update.simple_update, default schedule) and BP starts from the SU cells.  Returns this rank's rows."""
     if init not in ("random", "su"):
         raise ValueError(f"init must be 'random' or 'su', got {init!r}")
     mine = seeds_of_rank(list(seeds), rank, world)
@@ -89,7 +91,8 @@ def run_ensemble(seeds, D: int, N: int, chi_factor: float = 1.0, rank: int = 0, 
         from .simple_update import simple_update
         cells = [r.unit_cell for r in simple_update(cells, device=device)]
     res = belief_propagation_batch(N, cells, cfg, device=device, batch=batch)
-    rows = []
+    t_bp = time.perf_counter() - t0
+    done = []
     for s, cell, (msgs, its, err, ok) in zip(mine, cells, res):
         t1 = time.perf_counter()
         path = None
@@ -97,9 +100,15 @@ def run_ensemble(seeds, D: int, N: int, chi_factor: float = 1.0, rank: int = 0, 
             from .edge_env import EDGES
             cell, msgs, _, st = ite_flow.ite_edge_update(cell, msgs, N, "A", EDGES[k % 6], delta_t, cfg, chi, save=save_folder or False)
             path = st.saved_to or path
-        m = ite_flow.measure_energies(cell, msgs, N, chi)
+        done.append((s, cell, msgs, its, err, path, time.perf_counter() - t1))
+    # the energies of all the rank's cells: `batch` cells per launch of the compiled measurement
+    t2 = time.perf_counter()
+    ms = ite_flow.measure_energies_batch([x[1] for x in done], [x[2] for x in done], N, chi, device=device, batch=batch)
+    share = (t_bp + time.perf_counter() - t2) / max(1, len(mine))
+    rows = []
+    for (s, _, _, its, err, path, t_ite), m in zip(done, ms):
         rows.append({"seed": s, "D": D, "N": N, "chi": chi_factor, "energy": m.mean_energy, "parallel": world > 1, "path": path, "method": method,
-                     "exec_time": (time.perf_counter() - t1) + (t1 - t0) / max(1, len(mine)), "bp_iterations": its, "bp_error": err})
+                     "exec_time": t_ite + share, "bp_iterations": its, "bp_error": err})
     return rows
 
 

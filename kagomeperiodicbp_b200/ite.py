@@ -50,16 +50,25 @@ def _half_env(B, T, envs):
     return B.transpose(X, [0, 4, 1, 5, 2, 3])
 
 
-def rho_ij(B, Ti, Tj, mps_env):
-    """(ITE.py:683-756)  rho[i, i*, j, j*], trace normalised."""
+def rho_ij_unnormalized(B, Ti, Tj, mps_env):
+    """the contraction of ``rho_ij`` without its trace normalisation: rho[i, i*, j, j*] as a tensor of the backend ``B``.
+    Only backend operations, no host value: a compiled program can record it."""
     ni = Ti.ndim - 2
     Ai = _half_env(B, Ti, mps_env[:ni])                              # [p, p*, s, s*, L0, R_last]
     Aj = _half_env(B, Tj, mps_env[ni:])
     # ring closure: left bond of env_i[0] with right bond of env_j[-1], right bond of env_i[-1] with left bond of env_j[0]
-    rho = B.tensordot(Ai, Aj, ([2, 3, 4, 5], [2, 3, 5, 4]))
-    d = rho.shape[0]
-    tr = np.trace(np.trace(np.asarray(rho), axis1=0, axis2=1))       # scalar
-    return np.asarray(B.scale(rho, 1.0 / tr))
+    return B.tensordot(Ai, Aj, ([2, 3, 4, 5], [2, 3, 5, 4]))
+
+
+def rho_trace(rho) -> complex:
+    """trace of a two-site RDM rho[i, i*, j, j*] (a d^4 host reduction)."""
+    return np.trace(np.trace(np.asarray(rho), axis1=0, axis2=1))
+
+
+def rho_ij(B, Ti, Tj, mps_env):
+    """(ITE.py:683-756)  rho[i, i*, j, j*], trace normalised."""
+    rho = rho_ij_unnormalized(B, Ti, Tj, mps_env)
+    return np.asarray(B.scale(rho, 1.0 / rho_trace(rho)))
 
 
 def _n_half(B, T_rest, envs, n_legs):

@@ -7,6 +7,8 @@
 
 and the energy measurement ``measure_energies_and_observables_together`` (src/algo/measurements.py:163-243: six edge RDMs of
 one mode, energy per site = sum / 3).  Host code orchestrates and moves data; all tensor algebra runs through libkbp.so.
+``measure_energies_batch`` measures many unit cells at once: the reduction after the ToCore chains is shape-only, so it is
+compiled once (``compile_measurement``, recorded through ``linalg.TraceBackend``) and launched with one chain per cell.
 The core is reduced with bottom-up direction U unless told otherwise (the reference draws it at random from {U, DL, DR},
 kagome_to_core.py:178-179; SURVEY 8d fixes U for reproducible runs; `reduce_to_core(..., direction=)` takes all three).
 """
@@ -18,12 +20,16 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from . import belief_propagation as bp
-from . import edge_env, ite
+from . import edge_env, ite, linalg
 from .bubblecon import bubblecon as device_bubblecon
 from .containers import BPConfig, UnitCell
+from .dev_bubblecon import trace_bubblecon
+from .dev_mps import SLOT_NONFINITE
+from .engine import E_SVD_NOCONV, BubbleConError
 from .lattice import BLOCK_SIDES_CCW
-from .linalg import ResidentBackend
-from .runtime import get_engine
+from .linalg import ResidentBackend, TArr, TraceBackend
+from .program import Program
+from .runtime import Compiled, get_engine
 
 _backend = None
 
@@ -106,27 +112,173 @@ class MeasurementsOnUnitCell:
         return {k: sum(self.expectations[f][k] for f in "ABC") / 3 for k in "xyz"}
 
 
+def measurements_from_rdms(rdms: dict, flavors: dict, h) -> MeasurementsOnUnitCell:
+    """the host end of a measurement: energy, <sigma> and negativity of every edge from its trace-normalised two-site RDM.
+    ``rdms`` / ``flavors``: {edge: rho[i, i*, j, j*]} / {edge: (flavour of site i, flavour of site j)} in ``edge_env.EDGES``
+    order.  4 x 4 host arithmetic, as in the reference."""
+    energies, ent = {}, {}
+    acc = {f: {k: [0.0, 0] for k in "xyz"} for f in "ABC"}
+    for e, rho in rdms.items():
+        key = f"({e[0]}, {e[1]})"
+        energies[key] = float(np.real(np.dot(np.asarray(rho).flatten(), h.flatten())))
+        ent[key] = negativity_of_rdm(rho)
+        for k, vals in expectation_values_with_rdm(rho).items():
+            for v, f in zip(vals, flavors[e]):
+                acc[f][k][0] += v
+                acc[f][k][1] += 1
+    expectations = {f: {k: (acc[f][k][0] / acc[f][k][1] if acc[f][k][1] else 0.0) for k in "xyz"} for f in "ABC"}
+    return MeasurementsOnUnitCell(energies, dict(rdms), expectations, ent)
+
+
 def measure_energies(unit_cell: UnitCell, messages: dict, N: int, chi: int, h=None, mode: str = "A", env12=None) -> MeasurementsOnUnitCell:
     """(src/algo/measurements.py:163-243, energies part)"""
     h = ite.heisenberg_afm() if h is None else np.asarray(h)
     if env12 is None:
         env12 = reduce_to_core(unit_cell, messages, N, chi)
     B = backend()
-    energies, rdms, ent = {}, {}, {}
-    acc = {f: {k: [0.0, 0] for k in "xyz"} for f in "ABC"}
+    rdms, flavors = {}, {}
     for e in edge_env.EDGES:
         ti, tj, env, info = edge_tn(unit_cell, env12, N, mode, e, chi)
-        rho = ite.rho_ij(B, ti, tj, env)
-        rdms[e] = rho
-        key = f"({e[0]}, {e[1]})"
-        energies[key] = float(np.real(np.dot(np.asarray(rho).flatten(), h.flatten())))
-        ent[key] = negativity_of_rdm(rho)
-        for k, vals in expectation_values_with_rdm(rho).items():
-            for v, f in zip(vals, info["flavors"]):
-                acc[f][k][0] += v
-                acc[f][k][1] += 1
-    expectations = {f: {k: (acc[f][k][0] / acc[f][k][1] if acc[f][k][1] else 0.0) for k in "xyz"} for f in "ABC"}
-    return MeasurementsOnUnitCell(energies, rdms, expectations, ent)
+        rdms[e] = ite.rho_ij(B, ti, tj, env)
+        flavors[e] = info["flavors"]
+    return measurements_from_rdms(rdms, flavors, h)
+
+
+# ------------------------------------------------------------------------------------------------
+# the measurement of a batch of unit cells as one compiled program
+# ------------------------------------------------------------------------------------------------
+_measure_cache: dict = {}
+
+
+def compile_measurement(N: int, d: int, D: int, chi: int, mode: str, direction: str, tocore_shapes) -> Compiled:
+    """the whole measurement after the two ToCore chains as ONE program, compiled from shapes only: the zip of the two
+    boundary MPSs into the 12 ring tensors (``edge_env.core_env_tensors``), then for each of the six edges the Core -> Mode ->
+    Edge reduction (``edge_env.edge_environment``, its truncated ToEdge contractions recorded in place by ``trace_bubblecon``)
+    and the unnormalised two-site RDM (``ite.rho_ij_unnormalized``).  Every control decision of that code is shape-only and
+    the truncated SVDs decide per chain on the device, so one program serves any batch of cells.
+
+    ``tocore_shapes``: (site shapes of the bottom-up ToCore MPS, site shapes of the top-down one) of ``direction``.
+    Inputs: cellA, cellB, cellC [d, D, D, D, D], bu{k} and td{k} (the MPS sites).  Outputs: rho{k} [d, d, d, d] for the edges
+    of ``edge_env.EDGES``; slot SLOT_NONFINITE counts non-finite RDM entries.  meta["flavors"]: the site flavours per edge."""
+    bu_shapes, td_shapes = (tuple(tuple(int(x) for x in sh) for sh in side) for side in tocore_shapes)
+    key = (N, d, D, chi, mode, direction, bu_shapes, td_shapes)
+    if key in _measure_cache:
+        return _measure_cache[key]
+    p = Program(bp.N_SLOTS)
+    ins = [(nm, p.input(nm, (d, D, D, D, D))) for nm in ("cellA", "cellB", "cellC")]
+    ins += [(f"bu{k}", p.input(f"bu{k}", sh)) for k, sh in enumerate(bu_shapes)]
+    ins += [(f"td{k}", p.input(f"td{k}", sh)) for k, sh in enumerate(td_shapes)]
+    B = TraceBackend(p)
+    t = {nm: TArr(dt) for nm, dt in ins}
+    cell = (t["cellA"], t["cellB"], t["cellC"])
+    env12 = edge_env.core_env_tensors(B, N, [t[f"bu{k}"] for k in range(len(bu_shapes))],
+                                      [t[f"td{k}"] for k in range(len(td_shapes))], direction)
+
+    def bubblecon_fn(T_list, edges, angles, bubble_angle, order, D_trunc, kets):
+        # what compile_bubblecon records for the per-cell path, here inside the measurement program
+        mp, _ = trace_bubblecon(p, [x.dt for x in T_list], edges, angles, bubble_angle, list(order), D_trunc, kets)
+        return [TArr(x) for x in mp.dense_sites()]
+
+    outs, flavors = [], {}
+    for k, e in enumerate(edge_env.EDGES):
+        ti, tj, env, info = edge_env.edge_environment(B, N, cell, env12, mode, e, chi, bubblecon_fn)
+        rho = ite.rho_ij_unnormalized(B, ti, tj, env).dt
+        p.nonfinite(rho, SLOT_NONFINITE)
+        outs.append((f"rho{k}", rho))
+        flavors[e] = info["flavors"]
+    comp = Compiled(p, ins, outs, meta=dict(flavors=flavors))
+    _measure_cache[key] = comp
+    return comp
+
+
+def _measure_engine(device: int):
+    """the measurement program's own engine (stream + arena), from the pool the ITE backends use"""
+    return linalg.get_engine("measure", device)
+
+
+def _measure_chunk(cells, messages_list, index, N, chi, mode, direction, device):
+    """rdms ({edge: trace-normalised rho}) and flavours of the cells ``index`` (one shape group, one launch each)."""
+    bu_side, td_side, _ = edge_env.CORE_DIRECTIONS[direction]
+    d, D = cells[index[0]].A.shape[0], cells[index[0]].A.shape[1]
+    shapes = bp._msg_shapes(messages_list[index[0]])
+    futs = []
+    for side in (bu_side, td_side):
+        comp = bp.compile_side_program(N, d, D, side, chi, shapes, None, depth="ToCore", epilogue=False)
+        batch = [bp._side_inputs(cells[i], messages_list[i], comp) for i in index]
+        futs.append(bp._pool.submit(bp._run_side, side, comp, batch, device))
+    res = {}
+    for f in futs:
+        side, outs, slots, rc = f.result()
+        for c, i in enumerate(index):
+            if slots[c, -1] > 0:                   # engine status slot: a truncation of this chain did not converge
+                raise BubbleConError(f"cell {i}: truncated SVD did not converge in the ToCore contraction towards {side}")
+            if slots[c, bp.SLOT_NONFINITE] > 0:
+                raise BubbleConError(f"cell {i}: non-finite values in the ToCore contraction towards {side}")
+        res[side] = outs
+    n_bu, n_td = len(res[bu_side][0]), len(res[td_side][0])
+    comp = compile_measurement(N, d, D, chi, mode, direction,
+                               ([res[bu_side][0][f"out{k}"].shape for k in range(n_bu)],
+                                [res[td_side][0][f"out{k}"].shape for k in range(n_td)]))
+    batch = []
+    for c, i in enumerate(index):
+        x = {"cellA": cells[i].A, "cellB": cells[i].B, "cellC": cells[i].C}
+        x.update({f"bu{k}": res[bu_side][c][f"out{k}"] for k in range(n_bu)})
+        x.update({f"td{k}": res[td_side][c][f"out{k}"] for k in range(n_td)})
+        batch.append(x)
+    outs, slots, rc = comp.run(_measure_engine(device), batch, soft_errors=(E_SVD_NOCONV,))
+    rdms = []
+    for c, i in enumerate(index):
+        if slots[c, -1] > 0:
+            raise BubbleConError(f"cell {i}: truncated SVD did not converge in a ToEdge contraction of the measurement")
+        if slots[c, SLOT_NONFINITE] > 0:
+            raise BubbleConError(f"cell {i}: non-finite values in the measurement")
+        r = {}
+        for k, e in enumerate(edge_env.EDGES):
+            rho = outs[c][f"rho{k}"]
+            r[e] = rho * (1.0 / ite.rho_trace(rho))          # the trace normalisation of ite.rho_ij, on the host
+        rdms.append(r)
+    return rdms, comp.meta["flavors"]
+
+
+def measure_energies_batch(cells: list, messages_list: list, N: int, chi: int, h=None, mode: str = "A", direction: str = "U",
+                           device: int = 0, batch: int = 8) -> list:
+    """``measure_energies`` for a list of independent unit cells, ``batch`` cells per launch: cells with the same message
+    shapes share the two ToCore chains (run concurrently on their side engines) and one launch of the compiled measurement
+    program (``compile_measurement``); the host only normalises the RDMs and does the 4 x 4 arithmetic of every edge
+    (``measurements_from_rdms``).  -> [MeasurementsOnUnitCell] in input order.
+
+    Raises ValueError before any launch for an unknown ``mode`` / ``direction``, ``cells`` and ``messages_list`` of different
+    lengths, a non-repeated block (``LatticeTensors``) or cells of different d / D; BubbleConError naming the cell for a
+    truncation that did not converge or non-finite values."""
+    if len(cells) != len(messages_list):
+        raise ValueError(f"{len(cells)} cells but {len(messages_list)} message sets")
+    if mode not in edge_env.MODES:
+        raise ValueError(f"unknown mode {mode!r}: expected one of {edge_env.MODES}")
+    if direction not in edge_env.CORE_DIRECTIONS:
+        raise ValueError(f"unknown direction {direction!r}: expected one of {tuple(edge_env.CORE_DIRECTIONS)}")
+    if batch < 1:
+        raise ValueError(f"batch must be at least 1, got {batch}")
+    if not cells:
+        return []
+    for i, c in enumerate(cells):
+        if bp._is_arbitrary(c):
+            raise ValueError(f"cell {i} is a non-repeated block (LatticeTensors): the batched measurement takes unit cells")
+    d, D = cells[0].A.shape[0], cells[0].A.shape[1]
+    for i, c in enumerate(cells):
+        if any(t.shape != (d, D, D, D, D) for t in c.tensors()):
+            raise ValueError(f"cell {i} has tensors of shapes {[t.shape for t in c.tensors()]}, cell 0 has d = {d}, D = {D}")
+    h = ite.heisenberg_afm() if h is None else np.asarray(h)
+    groups: dict = {}
+    for i, m in enumerate(messages_list):
+        groups.setdefault(bp._msg_shapes(m), []).append(i)
+    out = [None] * len(cells)
+    for idx in groups.values():
+        for c0 in range(0, len(idx), batch):
+            chunk = idx[c0:c0 + batch]
+            rdms, flavors = _measure_chunk(cells, messages_list, chunk, N, chi, mode, direction, device)
+            for i, r in zip(chunk, rdms):
+                out[i] = measurements_from_rdms(r, flavors, h)
+    return out
 
 
 ENV_HERMICITY_THRESHOLD = 1e-4       # src/algo/imaginary_time_evolution/_constants.py

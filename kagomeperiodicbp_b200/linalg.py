@@ -313,3 +313,63 @@ class ResidentBackend:
         w = (s - _EIG_SHIFT) * nrm
         order = np.argsort(w, kind="stable")
         return w[order], np.conj(self.to_host(vh)[order]).T
+
+
+# ------------------------------------------------------------------------------------------------
+# tracing backend: the same algebra recorded into one compiled program, no host values at all
+# ------------------------------------------------------------------------------------------------
+class TArr:
+    """handle of a tensor recorded by a ``TraceBackend``: it has a shape but no value while the program is being built.
+    Converting it to numpy or indexing it raises, so host code that would need a value fails when the program is compiled,
+    not when it runs."""
+    __slots__ = ("dt",)
+
+    def __init__(self, dt):
+        self.dt = dt
+
+    shape = property(lambda self: self.dt.shape)
+    ndim = property(lambda self: self.dt.ndim)
+    size = property(lambda self: self.dt.size)
+
+    def __array__(self, dtype=None, copy=None):
+        raise TypeError(f"a traced tensor {self.shape} has no host value: the compiled program must not branch on data")
+
+    def __getitem__(self, idx):
+        raise TypeError(f"a traced tensor {self.shape} cannot be indexed on the host: reshape it through the backend")
+
+    def copy(self):
+        return self
+
+
+class TraceBackend:
+    """the backend interface of ``edge_env`` and ``ite.rho_ij_unnormalized`` (reshape, transpose, tensordot, qr) recorded into
+    the ``Program`` ``p``.  Every operand must be a ``TArr`` of that program (inputs are declared by the caller); there are no
+    scalar results, so nothing the trace does depends on data and the program replays for any batch of chains."""
+
+    def __init__(self, p: Program):
+        self.p = p
+
+    @staticmethod
+    def _dt(x):
+        if not isinstance(x, TArr):
+            raise TypeError(f"TraceBackend operand of type {type(x).__name__}: declare it as a program input")
+        return x.dt
+
+    def reshape(self, a, shape):
+        A = self._dt(a)
+        shape = tuple(int(s) for s in (shape if not isinstance(shape, int) else (shape,)))
+        if -1 in shape:
+            known = _prod(s for s in shape if s != -1)
+            shape = tuple(A.size // known if s == -1 else s for s in shape)
+        return TArr(A.reshape(shape))
+
+    def transpose(self, a, perm):
+        return TArr(self.p.transpose(self._dt(a), perm))
+
+    def tensordot(self, a, b, axes, conj_a=False, conj_b=False):
+        ax = (tuple(int(x) for x in axes[0]), tuple(int(x) for x in axes[1]))
+        return TArr(self.p.tensordot(self._dt(a), self._dt(b), ax, conj_a=conj_a, conj_b=conj_b))
+
+    def qr(self, m):
+        q, r = self.p.qr(self._dt(m))
+        return TArr(q), TArr(r)
